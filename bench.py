@@ -2,13 +2,15 @@
 
     python bench.py --gpus N --steps K --warmup W            # CUDA path (this repository)
     python bench.py --impl reference --gpus N ...            # the reference's own CPU code (oracle/_ref)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's result arrays to DIR
 
 A "step" = one pass of the hot path over one batch: every rank solves ``--batch`` synthetic 256x256 int8 constant
 matrices with the reference's default call (``solve(W)``: search over all decompose_dc candidates, two CSE stages each).
 Every step takes NEW matrices (seed + step); the steps whose matrices have a golden answer from the reference's own object
 code (tests/golden/index.json) are checked against it.  Matrices are independent, so ranks shard them with no data-path
 collective (weak scaling).  The line also carries a `c4` sub-record: BASELINE config 4, a fixed job of 64 128x128 int6
-matrices split over the ranks (strong scaling).  Prints ONE JSON line on rank 0.
+matrices split over the ranks (strong scaling).  Prints ONE JSON line on rank 0.  Writes nothing into the repository:
+figures it has to count at run time are cached in the temporary directory.
 """
 
 from __future__ import annotations
@@ -18,6 +20,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from pathlib import Path
@@ -26,6 +29,12 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # no __pycache__ in the tree for the modules imported from here on
+
+ALGO_BYTES = ROOT / 'profiles' / 'algo_bytes.json'  # committed figures
+ALGO_BYTES_RUN = Path(tempfile.gettempdir()) / 'da4ml_b200_bench' / 'algo_bytes.json'  # figures counted by earlier runs
+DUMP_LIMIT = 64 << 20  # bytes of --dump-outputs
+STAGE_KEYS = ('inp_shifts', 'out_idxs', 'out_shifts', 'out_negs', 'ops_i', 'ops_f')
 
 METRIC = 'cmvm_solve_throughput_256x256_int8'  # BASELINE.json metric (default workload)
 UNIT = 'matrices/s'
@@ -62,7 +71,7 @@ def stage_digest(stages) -> str:
 
     h = hashlib.sha256()
     for st in stages:
-        for k in ('inp_shifts', 'out_idxs', 'out_shifts', 'out_negs', 'ops_i', 'ops_f'):
+        for k in STAGE_KEYS:
             a = np.ascontiguousarray(st[k])
             h.update(k.encode())
             h.update(str(a.shape).encode())
@@ -118,19 +127,44 @@ def dist_env():
 
 
 def cached_algo_bytes(key: str):
-    cache = ROOT / 'profiles' / 'algo_bytes.json'
-    return json.loads(cache.read_text()).get(key) if cache.exists() else None
+    for cache in (ALGO_BYTES, ALGO_BYTES_RUN):
+        value = json.loads(cache.read_text()).get(key) if cache.exists() else None
+        if value is not None:
+            return value
+    return None
 
 
 def store_algo_bytes(key: str, value: float):
-    cache = ROOT / 'profiles' / 'algo_bytes.json'
-    known = json.loads(cache.read_text()) if cache.exists() else {}
-    known[key] = value
+    cache = ALGO_BYTES_RUN
     try:
-        cache.parent.mkdir(exist_ok=True)
-        cache.write_text(json.dumps(known, indent=1, sort_keys=True))
-    except OSError:
+        known = json.loads(cache.read_text()) if cache.exists() else {}
+        known[key] = value
+        cache.parent.mkdir(parents=True, exist_ok=True)
+        tmp = cache.with_suffix(f'.{os.getpid()}')
+        tmp.write_text(json.dumps(known, indent=1, sort_keys=True))
+        tmp.replace(cache)
+    except (OSError, ValueError):
         pass
+
+
+def dump_outputs(out_dir: Path, results, prefix: str, limit: int) -> None:
+    """The result arrays of one step (what solve_batch_device_raw hands its caller) as <out_dir>/<prefix>m<j>_s<i>_<key>.npy:
+    integers as float64 (exact), ops_f as float32.  Above ``limit`` bytes in all, every array keeps the same fraction of its
+    rows, drawn with a fixed seed."""
+    arrays = {}
+    for j, r in enumerate(results):
+        for i, st in enumerate(r.stages):
+            for k in STAGE_KEYS:
+                a = np.asarray(st[k])
+                arrays[f'{prefix}m{j}_s{i}_{k}'] = a.astype(np.float32 if a.dtype.kind == 'f' else np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    out_dir.mkdir(parents=True, exist_ok=True)
+    rng = np.random.default_rng(0)
+    for name, a in arrays.items():
+        if total > limit and len(a):
+            keep = max(1, int(len(a) * limit / total))
+            a = a[np.sort(rng.choice(len(a), keep, replace=False))]
+        np.save(out_dir / f'{name}.npy', a)
 
 
 def full_cpu_run(n: int, bits: int, seed: int = 0):
@@ -474,6 +508,9 @@ def run_cuda(args):
         full = full_cpu_run(n, bits, 0)
         if cpu is not None:
             line['cpu_baseline'] = {'value': cpu.get('value'), 'unit': UNIT, 'cores': cpu['cores'], 'kind': cpu['kind'], 'sample': cpu['sample'], 'algo_bytes_per_s': cpu['algo_bytes_per_s'], 'full_run_cached': full}
+    if args.dump_outputs:
+        dump_outputs(Path(args.dump_outputs), results[-1], f'rank{rank}_' if world > 1 else '', DUMP_LIMIT // world)
+    if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -495,7 +532,10 @@ def main():
     ap.add_argument('--c4', type=int, default=64, help='matrices of the BASELINE config 4 sub-record (128x128 int6, fixed job over the ranks); 0 disables')
     ap.add_argument('--cpu-seconds', type=float, default=15.0, help='bounded CPU-baseline sample (0 disables)')
     ap.add_argument('--recount', action='store_true', help='recompute the cached algorithmic-byte figures')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the result arrays of the last timed step to DIR/<name>.npy (CUDA arm)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
     return run_cuda(args)

@@ -1,3 +1,4 @@
+import hashlib
 import sys
 from pathlib import Path
 
@@ -30,6 +31,20 @@ def assert_stage_equal(a, b, tag=''):
             assert np.array_equal(x.view(np.uint32), y.astype(np.float32).view(np.uint32)), f'{tag}{k} differs'
         else:
             assert np.array_equal(x, y), f'{tag}{k} differs'
+
+
+def digest(named_arrays):
+    """SHA-256 over (name, dtype, shape, bytes) of each array: how a golden file stores an answer it does not keep whole."""
+    h = hashlib.sha256()
+    for name, a in named_arrays:
+        a = np.ascontiguousarray(a)
+        h.update(f'{name} {a.dtype.str} {a.shape}'.encode())
+        h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def stage_digest(stages):
+    return digest((f's{i}_{k}', st[k]) for i, st in enumerate(stages) for k in STAGE_KEYS)
 
 
 def golden_cases(full_only=True):

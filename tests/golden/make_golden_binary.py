@@ -1,7 +1,7 @@
 """DAIS binary golden vectors from the reference's own ``da4ml.types.CombLogic.to_binary`` (types.py:500-541).
 
-Container only: imports /root/reference/src/da4ml/types.py with a stub standing in for its native module (the reference
-package itself cannot be installed here: meson/nanobind/xtensor are absent).  Writes tests/golden/dais_binary.npz.
+Imports types.py of the da4ml source tree oracle/_ref is built from (tests/ref_trace.py) with a stub standing in for its
+native module (the reference package itself needs meson/nanobind/xtensor to install).  Writes tests/golden/dais_binary.npz.
 """
 import importlib.util
 import sys
@@ -16,13 +16,15 @@ sys.path.insert(0, str(HERE.parent))
 
 
 def reference_types():
+    from ref_trace import REF
+
     pkg = types.ModuleType('da4ml')
-    pkg.__path__ = ['/root/reference/src/da4ml']
+    pkg.__path__ = [REF]
     sys.modules['da4ml'] = pkg
     stub = types.ModuleType('da4ml._binary')
     stub.dais_interp_run = lambda *a, **k: None
     sys.modules['da4ml._binary'] = stub
-    spec = importlib.util.spec_from_file_location('da4ml.types', '/root/reference/src/da4ml/types.py')
+    spec = importlib.util.spec_from_file_location('da4ml.types', f'{REF}/types.py')
     T = importlib.util.module_from_spec(spec)
     sys.modules['da4ml.types'] = T
     spec.loader.exec_module(T)

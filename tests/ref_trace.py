@@ -1,11 +1,20 @@
-"""Import the reference's pure-Python ``da4ml.trace`` package (container only: /root/reference) with its native module
-``da4ml._binary`` replaced by a stand-in built from callables the test supplies -- the way an integration would point the
-tracing front-end at another solver.  TEST INFRASTRUCTURE."""
+"""Import the reference's pure-Python ``da4ml.trace`` package (from the da4ml source tree oracle/_ref was built from, as
+recorded in oracle/_ref/source_tree by `make -C oracle`) with its native module ``da4ml._binary`` replaced by a stand-in
+built from callables the test supplies -- the way an integration would point the tracing front-end at another solver.
+TEST INFRASTRUCTURE."""
 import importlib
+import os
 import sys
 import types
+from pathlib import Path
 
-REF = '/root/reference/src/da4ml'
+_RECORD = Path(__file__).resolve().parents[1] / 'oracle' / '_ref' / 'source_tree'
+REF = os.path.join(_RECORD.read_text().strip(), 'src', 'da4ml') if _RECORD.is_file() else None
+
+
+def available() -> bool:
+    """The reference's Python sources can be read (isdir is False for a missing or unreadable tree)."""
+    return REF is not None and os.path.isdir(os.path.join(REF, 'trace'))
 
 
 def load(solve, get_lsb_loc, iceil_log2, cost_add, kernel_decompose=None, csd_decompose=None, int_arr_to_csd=None):

@@ -4,6 +4,8 @@ import subprocess
 import sys
 from pathlib import Path
 
+import numpy as np
+
 ROOT = Path(__file__).resolve().parents[1]
 
 
@@ -29,3 +31,31 @@ def test_default_metric_is_the_baseline_metric():
     assert bench.metric_name(256, 8) == bench.METRIC == 'cmvm_solve_throughput_256x256_int8'
     spec = json.loads((ROOT / 'BASELINE.json').read_text())
     assert '256' in spec['metric'] and 'int8' in spec['metric']
+
+
+def test_dump_outputs_writes_result_arrays_as_float(tmp_path):
+    """--dump-outputs: every result array of the step as float64 (integers) / float32 (ops_f); above the byte limit the
+    same seeded sample of rows in every run."""
+    sys.path.insert(0, str(ROOT))
+    from types import SimpleNamespace
+
+    import bench
+    from conftest import load_golden
+
+    _, stages = load_golden('int_32x32_int8_default')
+    step = [SimpleNamespace(stages=stages)]
+    bench.dump_outputs(tmp_path / 'all', step, '', bench.DUMP_LIMIT)
+    for i, st in enumerate(stages):
+        for k in bench.STAGE_KEYS:
+            a = np.load(tmp_path / 'all' / f'm0_s{i}_{k}.npy')
+            assert a.dtype == (np.float32 if k == 'ops_f' else np.float64)
+            assert np.array_equal(a, st[k]), k
+    limit = sum(np.asarray(st[k]).size * 8 for st in stages for k in bench.STAGE_KEYS) // 4
+    for run in ('a', 'b'):
+        bench.dump_outputs(tmp_path / run, step, 'x_', limit)
+    files = sorted(p.name for p in (tmp_path / 'a').iterdir())
+    assert len(files) == 2 * len(bench.STAGE_KEYS) and sum((tmp_path / 'a' / f).stat().st_size for f in files) < limit + 128 * len(files)
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / 'a' / f), np.load(tmp_path / 'b' / f))
+    ops = np.load(tmp_path / 'a' / 'x_m0_s0_ops_i.npy')
+    assert 0 < len(ops) < len(stages[0]['ops_i']) and all(any((row == o).all() for o in stages[0]['ops_i']) for row in ops)

@@ -1,14 +1,19 @@
 """SURVEY 8f N2: replay of the adder graphs with the DAIS int64 semantics.  CPU: the compiled reference interpreter
 (oracle/_ref/libdais_ref.so) agrees with the float replay on in-range inputs.  GPU: the CUDA replay equals the reference
-interpreter bit for bit, including the wrap-around of out-of-range inputs."""
+interpreter bit for bit, including the wrap-around of out-of-range inputs.  The interpreter's answers (a digest for the
+largest) are stored in tests/golden/dais_ref.npz (written by tests/golden/make_golden_ref_outputs.py)."""
+import hashlib
+
 import numpy as np
 import pytest
-from conftest import golden_cases, int_matrix, load_golden
+from conftest import GOLDEN, digest, golden_cases, int_matrix, load_golden
 
 from da4ml_b200.types import pipeline_from_arrays
-from oracle import dais_ref
 
-needs_ref = pytest.mark.skipif(not dais_ref.available(), reason='oracle/_ref/libdais_ref.so not built')
+
+@pytest.fixture(scope='module')
+def gold():
+    return np.load(GOLDEN / 'dais_ref.npz')
 
 
 def golden_stage_programs():
@@ -23,37 +28,58 @@ def golden_stage_programs():
     return out
 
 
-@needs_ref
-def test_reference_interpreter_agrees_with_float_replay():
+def float_replay_inputs():
+    """(tag, program, samples): stage-0 graphs with the default 8-bit inputs, every sample in range."""
     rng = np.random.default_rng(0)
     for tag, sol in golden_stage_programs():
         if '/s0' not in tag or 'hetero' in tag:
-            continue  # stage-0 graphs with the default 8-bit inputs: every sample is in range
-        x = rng.integers(-128, 128, size=(9, sol.shape[0])).astype(np.float64)
-        assert np.array_equal(dais_ref.run(sol.to_binary(), x), sol(x)), tag
+            continue
+        yield tag, sol, rng.integers(-128, 128, size=(9, sol.shape[0])).astype(np.float64)
 
 
-@needs_ref
-@pytest.mark.gpu
-def test_cuda_replay_matches_reference_interpreter(cuda_binary):
+def cuda_replay_inputs():
+    """(tag, program, samples): every golden stage, in-range samples and out-of-range ones that wrap around."""
     rng = np.random.default_rng(1)
     for tag, sol in golden_stage_programs():
         n_in = sol.shape[0]
-        x = np.concatenate([rng.integers(-128, 128, size=(33, n_in)), rng.integers(-5000, 5000, size=(8, n_in)) / 8.0]).astype(np.float64)
-        want = dais_ref.run(sol.to_binary(), x)
+        yield tag, sol, np.concatenate([rng.integers(-128, 128, size=(33, n_in)), rng.integers(-5000, 5000, size=(8, n_in)) / 8.0]).astype(np.float64)
+
+
+SOLVED_KW = dict(search_all_decompose_dc=False, decompose_dc=-1)
+
+
+def solved_matrix_case():
+    return int_matrix(64, 48, 8, 21), np.random.default_rng(2).integers(-128, 128, size=(5000, 64)).astype(np.float64)
+
+
+def call_key(prog, x):
+    """Name under which the interpreter's answer to one call (program, samples) is stored."""
+    h = hashlib.sha256(np.ascontiguousarray(prog, dtype=np.int32).tobytes())
+    h.update(np.ascontiguousarray(x, dtype=np.float64).tobytes())
+    return 'call_' + h.hexdigest()[:32]
+
+
+def test_reference_interpreter_agrees_with_float_replay(gold):
+    for tag, sol, x in float_replay_inputs():
+        assert np.array_equal(gold['float__' + tag.replace('/', '__')], sol(x)), tag
+
+
+@pytest.mark.gpu
+def test_cuda_replay_matches_reference_interpreter(cuda_binary, gold):
+    for tag, sol, x in cuda_replay_inputs():
+        want = gold['cuda__' + tag.replace('/', '__')]
         got = sol.predict(x)
         assert got.dtype == np.float64 and np.array_equal(got.view(np.uint64), want.view(np.uint64)), tag
 
 
-@needs_ref
 @pytest.mark.gpu
-def test_cuda_replay_of_a_solved_matrix(cuda_binary):
-    W = int_matrix(64, 48, 8, 21)
-    pipe = cuda_binary.solve(W, search_all_decompose_dc=False, decompose_dc=-1)
+def test_cuda_replay_of_a_solved_matrix(cuda_binary, gold):
+    W, x = solved_matrix_case()
+    pipe = cuda_binary.solve(W, **SOLVED_KW)
     sol = pipe.solutions[0]
-    x = np.random.default_rng(2).integers(-128, 128, size=(5000, 64)).astype(np.float64)
+    assert digest([('program', sol.to_binary())]) == str(gold['solved_program'])  # the program the stored answer belongs to
     got = sol.predict(x)
-    assert np.array_equal(got, dais_ref.run(sol.to_binary(), x))
+    assert digest([('out', got)]) == str(gold['solved_out'])
     assert np.array_equal(got, sol(x))  # in-range inputs: fixed-point replay == exact arithmetic
     with pytest.raises(RuntimeError, match='Unknown opcode'):
         bad = sol.to_binary()
@@ -74,13 +100,18 @@ def _raw_from_golden(name):
     return B.RawPipeline.from_stages(stages), want
 
 
-@needs_ref
-def test_kernel_from_fixed_point_probes(monkeypatch):
+def test_kernel_from_fixed_point_probes(monkeypatch, gold):
     """``RawPipeline.kernel`` probes every stage with one quantum per input under the DAIS fixed-point semantics; with
-    the reference interpreter standing in for the CUDA one, it reproduces the matrix of every golden case."""
+    the reference interpreter standing in for the CUDA one (its stored answers to exactly these probes), it reproduces
+    the matrix of every golden case."""
     import da4ml_b200._binary as B
 
-    monkeypatch.setattr(B, 'dais_interp_run', lambda prog, x, n_threads=1: dais_ref.run(prog, x))
+    def reference_answer(prog, x, n_threads=1):
+        key = call_key(prog, x)
+        assert key in gold.files, 'a probe the reference interpreter was not asked when the golden file was made'
+        return gold[key].copy()
+
+    monkeypatch.setattr(B, 'dais_interp_run', reference_answer)
     for name in golden_cases():
         raw, want = _raw_from_golden(name)
         assert np.array_equal(raw.kernel, want), name

@@ -192,7 +192,7 @@ def test_retiming_matches_the_reference_tracer(gold, name):
     assert n_checked > 0
 
 
-@pytest.mark.skipif(not __import__('pathlib').Path('/root/reference/src/da4ml/trace').exists(), reason='needs the reference tree (build container)')
+@pytest.mark.skipif(not __import__('ref_trace').available(), reason='needs the da4ml source tree oracle/_ref is built from')
 def test_retiming_is_delegated_to_the_reference_tracer():
     """``retiming=True, da4ml=<package>`` hands the split to the reference's own ``retime_pipeline`` and returns flat stages
     (the route for graphs in which the tracer produces constants); equal to the reference's ``to_pipeline(..., retiming=True)``

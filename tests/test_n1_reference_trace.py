@@ -1,16 +1,15 @@
 """SURVEY 8f N1, reference side (CPU, build container only): the reference's own ``da4ml.trace.FixedVariableArray.matmul``
-(trace/fixed_variable_array.py:333-373) is imported from /root/reference with its native module replaced by a stand-in
+(trace/fixed_variable_array.py:333-373) is imported from the reference tree with its native module replaced by a stand-in
 (tests/ref_trace.py) and pointed at ``SolveBatcher.solve``.  Checks that the two-pass batching is transparent to the real
 front-end: the same calls in the same order in both passes, one batched solve, and the traced result of the second pass
 equals what the front-end builds call by call.  The solver here is the CPU checker (the CUDA solver needs a GPU; the GPU
 suite checks the batched CUDA path against the checker, tests/test_n1_traced_matmul_gpu.py)."""
-from pathlib import Path
-
 import numpy as np
 import pytest
+import ref_trace
 from conftest import int_matrix
 
-pytestmark = pytest.mark.skipif(not Path('/root/reference/src/da4ml/trace').exists(), reason='needs the reference tree (build container)')
+pytestmark = pytest.mark.skipif(not ref_trace.available(), reason='needs the da4ml source tree oracle/_ref is built from')
 
 
 def _checker_batch(types_module):
@@ -33,8 +32,6 @@ def _checker_batch(types_module):
 
 
 def test_reference_matmul_through_the_batcher():
-    import ref_trace
-
     import da4ml_b200._binary as B
     from da4ml_b200.batching import SolveBatcher
 

@@ -1,13 +1,14 @@
 """The independent restatement (oracle/port) against the reference's own object code (oracle/_ref) on a broad random
 family of inputs: ragged shapes, sparse / scaled / wide matrices, heterogeneous intervals and latencies, every
-selector.  This is what lets the port stand in as the checker on a box where oracle/_ref is absent.  No GPU."""
+selector.  This is what lets the port stand in as the checker wherever oracle/_ref is absent.  The reference's answers
+are stored as digests in tests/golden/oracle_digests.json (written by tests/golden/make_golden_ref_outputs.py).  No GPU."""
+import json
+
 import numpy as np
 import pytest
-from conftest import assert_stage_equal
+from conftest import GOLDEN, digest, stage_digest
 
-from oracle import port, ref
-
-pytestmark = pytest.mark.skipif(not ref.available(), reason='oracle/_ref not built (needs /root/reference)')
+from oracle import port
 
 METHODS = ['mc', 'wmc', 'mc-dc', 'mc-pdc', 'wmc-dc', 'wmc-pdc']
 
@@ -64,8 +65,7 @@ def shapes(rng):
     return int(rng.integers(2, 22)), int(rng.integers(2, 22))
 
 
-@pytest.mark.parametrize('seed', range(60))
-def test_single_stage_random_family(seed):
+def single_case(seed):
     rng = np.random.default_rng(7000 + seed)
     n_in, n_out = shapes(rng)
     W, kind = random_matrix(rng, n_in, n_out)
@@ -76,11 +76,10 @@ def test_single_stage_random_family(seed):
         adder_size=int(rng.choice([-1, 1, 3, 8])),
         carry_size=int(rng.choice([-1, 1, 4])),
     )
-    assert_stage_equal(ref.solve_single(W, **kw), port.solve_single(W, **kw), f'{kind} {W.shape} {kw["method"]} ')
+    return W, kind, kw
 
 
-@pytest.mark.parametrize('seed', range(40))
-def test_full_solve_random_family(seed):
+def full_case(seed):
     rng = np.random.default_rng(9000 + seed)
     n_in, n_out = shapes(rng)
     W, kind = random_matrix(rng, n_in, n_out)
@@ -95,25 +94,62 @@ def test_full_solve_random_family(seed):
         carry_size=int(rng.choice([-1, 3])),
         search_all_decompose_dc=bool(rng.integers(0, 2)),
     )
-    a, b = ref.solve(W, **kw), port.solve(W, **kw)
-    assert len(a) == len(b) == 2
-    for i, (x, y) in enumerate(zip(a, b)):
-        assert_stage_equal(x, y, f'{kind} {W.shape} {kw} stage{i} ')
+    return W, kind, kw
 
 
-@pytest.mark.parametrize('seed', range(20))
-def test_helpers_random_family(seed):
+def helpers_case(seed):
     rng = np.random.default_rng(11000 + seed)
     n_in, n_out = shapes(rng)
     W, _ = random_matrix(rng, n_in, n_out)
-    for center in (True, False):
-        a, b = ref.csd_decompose(W, center), port.csd_decompose(W, center)
-        for x, y in zip(a, b):
-            assert x.shape == y.shape and np.array_equal(x, y)
     ints = rng.integers(-(2**20), 2**20, size=(int(rng.integers(1, 40)),)).astype(np.int32)
-    assert np.array_equal(ref.int_arr_to_csd(ints), port.int_arr_to_csd(ints))
     Wi = np.round(W * 64).astype(np.float32)  # kernel_decompose works on the integer grid
-    for dc in (-2, -1, 0, 1, 2):
-        a, b = ref.kernel_decompose(Wi, dc), port.kernel_decompose(Wi, dc)
-        assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), dc
-        assert np.array_equal(a[0].astype(np.float64) @ a[1].astype(np.float64), Wi)
+    return W, ints, Wi
+
+
+DECOMPOSE_DCS = (-2, -1, 0, 1, 2)
+
+
+def helpers_outputs(mod, W, ints, Wi):
+    """Every helper's arrays for one case, under the names the golden file stores them."""
+    out = {}
+    for center in (True, False):
+        for name, a in zip(('csd', 's0', 's1'), mod.csd_decompose(W, center)):
+            out[f'csd{int(center)}_{name}'] = a
+    out['int_csd'] = mod.int_arr_to_csd(ints)
+    for dc in DECOMPOSE_DCS:
+        out[f'kd{dc}_m0'], out[f'kd{dc}_m1'] = mod.kernel_decompose(Wi, dc)
+    return out
+
+
+@pytest.fixture(scope='module')
+def gold():
+    return json.loads((GOLDEN / 'oracle_digests.json').read_text())
+
+
+@pytest.mark.parametrize('seed', range(60))
+def test_single_stage_random_family(gold, seed):
+    W, kind, kw = single_case(seed)
+    g = gold[f'single{seed}']
+    assert digest([('kernel', W)]) == g['kernel'], 'not the matrix the reference answered for'
+    assert stage_digest([port.solve_single(W, **kw)]) == g['result'], f'{kind} {W.shape} {kw["method"]}: differs from the reference'
+
+
+@pytest.mark.parametrize('seed', range(40))
+def test_full_solve_random_family(gold, seed):
+    W, kind, kw = full_case(seed)
+    g = gold[f'full{seed}']
+    assert digest([('kernel', W)]) == g['kernel'], 'not the matrix the reference answered for'
+    got = port.solve(W, **kw)
+    assert len(got) == 2
+    assert stage_digest(got) == g['result'], f'{kind} {W.shape} {kw}: differs from the reference'
+
+
+@pytest.mark.parametrize('seed', range(20))
+def test_helpers_random_family(gold, seed):
+    W, ints, Wi = helpers_case(seed)
+    g = gold[f'helpers{seed}']
+    assert digest([('kernel', W)]) == g['kernel'], 'not the matrix the reference answered for'
+    got = helpers_outputs(port, W, ints, Wi)
+    assert digest(sorted(got.items())) == g['result'], 'differs from the reference'
+    for dc in DECOMPOSE_DCS:
+        assert np.array_equal(got[f'kd{dc}_m0'].astype(np.float64) @ got[f'kd{dc}_m1'].astype(np.float64), Wi), dc

@@ -80,14 +80,13 @@ def test_serialisers_from_flat_arrays_match_the_container_path(tmp_path):
 
 
 def test_results_build_the_reference_own_containers():
-    """Drop-in check (container only): with ``types_module=da4ml.types`` the result is made of the reference's own
-    NamedTuples, as its nanobind glue does (bindings.cc:106-151), and its serialiser accepts them."""
-    import os
-
+    """Drop-in check (needs the reference tree): with ``types_module=da4ml.types`` the result is made of the reference's
+    own NamedTuples, as its nanobind glue does (bindings.cc:106-151), and its serialiser accepts them."""
     import pytest
+    import ref_trace
 
-    if not os.path.exists('/root/reference/src/da4ml/types.py'):
-        pytest.skip('reference tree not present')
+    if not ref_trace.available():
+        pytest.skip('needs the da4ml source tree oracle/_ref is built from')
     import sys
 
     sys.path.insert(0, str(__import__('pathlib').Path(__file__).resolve().parent / 'golden'))
