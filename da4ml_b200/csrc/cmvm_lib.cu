@@ -6,6 +6,7 @@
 // candidates (and of all problems of a batch) are solved concurrently by one persistent kernel
 // launch per round.  All arithmetic of the path runs in the kernels of cmvm_kernels.cuh /
 // cmvm_decompose.cuh; nothing here falls back to the CPU.
+#include "host_dais.cuh"
 #include "host_solve.cuh"
 
 namespace da {
@@ -55,6 +56,71 @@ using namespace da;
 struct da4ml_pipeline {
     std::unique_ptr<PipelineImpl> impl;
 };
+
+// A DAIS program compiled for the device and kept resident (host_dais.cuh, dais_exec.cuh).
+struct da4ml_dais {
+    DaisCompiled P;
+    int device = -1;
+    int tile = 0;           // samples per CTA in the shared regime; 0 = global regime
+    long long chunk = 0;    // samples per launch
+    bool has_lookup = false;
+    void *mem = nullptr;    // instructions | tables | error word, v0 word
+    DaisInstr *d_prog = nullptr;
+    int32_t *d_tables = nullptr;
+    unsigned long long *d_err = nullptr;
+    long long *d_v0 = nullptr;
+    ~da4ml_dais() {
+        if (mem)
+            cudaFree(mem);
+    }
+};
+
+namespace {
+long long g_dais_shared_budget = 0; // bytes of shared memory for one CTA's slot file; 0 = what the device allows
+long long g_dais_chunk = 0;         // samples per launch; 0 = automatic
+DevBuf g_dais_arena, g_dais_io;
+
+void dais_launch(const da4ml_dais *h, const double *x, double *y, long long n, long long sample0, unsigned long long *err, long long *err_v0) {
+    const DaisCompiled &P = h->P;
+    const int n_instr = (int)P.prog.size();
+    if (h->tile > 0) {
+        const size_t smem = (size_t)8 * std::max(P.n_slots, 1) * h->tile;
+        dais_exec_kernel<true><<<(unsigned)((n + h->tile - 1) / h->tile), h->tile, smem, g_stream>>>(h->d_prog, n_instr, x, P.n_in, y, P.n_out, n, nullptr, 0, h->d_tables, err, sample0, err_v0);
+    }
+    else {
+        g_dais_arena.ensure((size_t)8 * std::max(P.n_slots, 1) * std::max(n, 1LL), false);
+        dais_exec_kernel<false><<<(unsigned)((n + 255) / 256), 256, 0, g_stream>>>(h->d_prog, n_instr, x, P.n_in, y, P.n_out, n, (long long *)g_dais_arena.p, n, h->d_tables, err, sample0, err_v0);
+    }
+    CK(cudaGetLastError());
+}
+
+// After the launches of a call: raise the reference's message for the first (sample, op) whose lookup was out of range.
+// That sample is run once more on its own to recover the operand.  `row(s)` is a device pointer to input row s.
+template <class Row> void dais_check(const da4ml_dais *h, Row row, double *y_scratch) {
+    if (!h->has_lookup)
+        return;
+    unsigned long long key = 0;
+    CK(cudaMemcpyAsync(&key, h->d_err, sizeof(key), cudaMemcpyDeviceToHost, g_stream));
+    CK(cudaStreamSynchronize(g_stream));
+    if (key == ~0ull)
+        return;
+    const unsigned long long n_instr = h->P.prog.size();
+    const long long s = (long long)(key / n_instr);
+    const int pc = (int)(key % n_instr);
+    dais_launch(h, row(s), y_scratch, 1, 0, h->d_err + 1, h->d_v0);
+    long long v0 = 0;
+    CK(cudaMemcpyAsync(&v0, h->d_v0, sizeof(v0), cudaMemcpyDeviceToHost, g_stream));
+    CK(cudaStreamSynchronize(g_stream));
+    throw ApiError(DA4ML_E_RUNTIME, dais_lookup_message(h->P, pc, v0));
+}
+
+void dais_check_device(const da4ml_dais *h) {
+    int dev = 0;
+    CK(cudaGetDevice(&dev));
+    if (dev != h->device)
+        throw ApiError(DA4ML_E_INVALID, "the DAIS program was loaded on CUDA device " + std::to_string(h->device) + ", the current device is " + std::to_string(dev));
+}
+} // namespace
 
 template <class F> static int guarded(F &&f) {
     try {
@@ -532,6 +598,127 @@ int da4ml_dais_run(const int32_t *program, int64_t n_words, const double *inputs
             CK(cudaStreamSynchronize(g_stream));
         }
     });
+}
+
+// ---- complete DAIS interpreter: programs loaded once and kept on the device -----------------------------------------
+int da4ml_dais_set_shared_budget(int64_t shared_bytes, int64_t chunk_samples) {
+    g_dais_shared_budget = std::max<int64_t>(shared_bytes, 0);
+    g_dais_chunk = std::max<int64_t>(chunk_samples, 0);
+    return DA4ML_OK;
+}
+
+int da4ml_dais_load(const int32_t *program, int64_t n_words, da4ml_dais_t **out) {
+    return guarded([&] {
+        if (!out)
+            throw ApiError(DA4ML_E_INVALID, "invalid argument");
+        auto h = std::make_unique<da4ml_dais>();
+        try {
+            h->P = dais_compile(program, n_words);
+        }
+        catch (const std::runtime_error &e) {
+            throw ApiError(DA4ML_E_RUNTIME, e.what());
+        }
+        init_device();
+        h->device = g_device;
+        const DaisCompiled &P = h->P;
+        for (const DaisInstr &I : P.prog)
+            h->has_lookup |= I.kind == DK_LOOKUP;
+        int optin = 0;
+        CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, g_device));
+        const long long budget = g_dais_shared_budget > 0 ? std::min<long long>(g_dais_shared_budget, optin) : optin;
+        h->tile = dais_shared_tile(P.n_slots, budget);
+        if (h->tile > 0) {
+            CK(cudaFuncSetAttribute(dais_exec_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+            h->chunk = 1LL << 24; // (bounds the staging buffers of host arrays)
+        }
+        else
+            h->chunk = std::max<long long>(256, ((1LL << 31) / (8LL * P.n_slots)) / 256 * 256); // a 2 GB slot arena
+        h->chunk = std::min<long long>(h->chunk, std::max<long long>(256, ((1LL << 28) / (8LL * std::max(1, P.n_in + P.n_out))) / 256 * 256));
+        if (g_dais_chunk > 0)
+            h->chunk = g_dais_chunk;
+        Carver c;
+        const size_t o_prog = c.take(sizeof(DaisInstr) * P.prog.size()), o_tab = c.take(sizeof(int32_t) * P.tables.size()), o_err = c.take(4 * sizeof(long long));
+        CK(cudaMalloc(&h->mem, c.off));
+        h->d_prog = (DaisInstr *)((char *)h->mem + o_prog);
+        h->d_tables = (int32_t *)((char *)h->mem + o_tab);
+        h->d_err = (unsigned long long *)((char *)h->mem + o_err);
+        h->d_v0 = (long long *)(h->d_err + 2);
+        CK(cudaMemcpyAsync(h->d_prog, P.prog.data(), sizeof(DaisInstr) * P.prog.size(), cudaMemcpyHostToDevice, g_stream));
+        if (!P.tables.empty())
+            CK(cudaMemcpyAsync(h->d_tables, P.tables.data(), sizeof(int32_t) * P.tables.size(), cudaMemcpyHostToDevice, g_stream));
+        CK(cudaStreamSynchronize(g_stream));
+        *out = h.release();
+    });
+}
+
+int da4ml_dais_info(const da4ml_dais_t *h, int64_t out[8]) {
+    if (!h || !out)
+        return DA4ML_E_INVALID;
+    const DaisCompiled &P = h->P;
+    out[0] = P.n_in;
+    out[1] = P.n_out;
+    out[2] = P.n_ops;
+    out[3] = P.n_tables;
+    out[4] = P.n_slots;
+    out[5] = h->tile > 0 ? 0 : 1;
+    out[6] = h->tile > 0 ? h->tile : h->chunk;
+    out[7] = P.max_width;
+    return DA4ML_OK;
+}
+
+int da4ml_dais_infer(da4ml_dais_t *h, const double *x, int64_t n_samples, double *y) {
+    return guarded([&] {
+        if (!h || n_samples < 0 || (n_samples > 0 && ((!x && h->P.n_in) || (!y && h->P.n_out))))
+            throw ApiError(DA4ML_E_INVALID, "invalid argument");
+        if (n_samples == 0)
+            return;
+        init_device();
+        dais_check_device(h);
+        const DaisCompiled &P = h->P;
+        const long long C = std::min<long long>(h->chunk, n_samples);
+        Carver c;
+        const size_t o_x = c.take(sizeof(double) * std::max<long long>(C * P.n_in, 1)), o_y = c.take(sizeof(double) * std::max<long long>(C * P.n_out, 1));
+        g_dais_io.ensure(c.off, false);
+        double *dx = (double *)((char *)g_dais_io.p + o_x), *dy = (double *)((char *)g_dais_io.p + o_y);
+        CK(cudaMemsetAsync(h->d_err, 0xff, 2 * sizeof(unsigned long long), g_stream));
+        for (long long s0 = 0; s0 < n_samples; s0 += C) {
+            const long long Sc = std::min<long long>(C, n_samples - s0);
+            if (P.n_in)
+                CK(cudaMemcpyAsync(dx, x + s0 * P.n_in, sizeof(double) * Sc * P.n_in, cudaMemcpyHostToDevice, g_stream));
+            dais_launch(h, dx, dy, Sc, s0, h->d_err, nullptr);
+            dais_check(h, [&](long long s) {
+                CK(cudaMemcpyAsync(dx, x + s * P.n_in, sizeof(double) * P.n_in, cudaMemcpyHostToDevice, g_stream));
+                return (const double *)dx;
+            }, dy);
+            if (P.n_out)
+                CK(cudaMemcpyAsync(y + s0 * P.n_out, dy, sizeof(double) * Sc * P.n_out, cudaMemcpyDeviceToHost, g_stream));
+            CK(cudaStreamSynchronize(g_stream));
+        }
+    });
+}
+
+int da4ml_dais_infer_device(da4ml_dais_t *h, const double *x_dev, int64_t n_samples, double *y_dev) {
+    return guarded([&] {
+        if (!h || n_samples < 0 || (n_samples > 0 && ((!x_dev && h->P.n_in) || (!y_dev && h->P.n_out))))
+            throw ApiError(DA4ML_E_INVALID, "invalid argument");
+        if (n_samples == 0)
+            return;
+        init_device();
+        dais_check_device(h);
+        const DaisCompiled &P = h->P;
+        g_dais_io.ensure(sizeof(double) * std::max(P.n_out, 1), false);
+        CK(cudaMemsetAsync(h->d_err, 0xff, 2 * sizeof(unsigned long long), g_stream));
+        for (long long s0 = 0; s0 < n_samples; s0 += h->chunk) {
+            const long long Sc = std::min<long long>(h->chunk, n_samples - s0);
+            dais_launch(h, x_dev + s0 * P.n_in, y_dev + s0 * P.n_out, Sc, s0, h->d_err, nullptr);
+        }
+        dais_check(h, [&](long long s) { return x_dev + s * P.n_in; }, (double *)g_dais_io.p);
+    });
+}
+
+void da4ml_dais_free(da4ml_dais_t *h) {
+    std::lock_guard<std::mutex> lock(g_mutex);
+    delete h;
 }
 
 int da4ml_cmvm_get_lsb_loc(float x) { return get_lsb_loc(x); }

@@ -137,6 +137,25 @@ int da4ml_pipeline_profile(const da4ml_pipeline_t *p, double out[8]);
  * Bit-exact int64 fixed-point semantics of the reference interpreter. */
 int da4ml_dais_run(const int32_t *program, int64_t n_words, const double *inputs, int64_t n_samples, double *outputs);
 
+/* ---- complete DAIS interpreter ---------------------------------------------------------------------
+ * Every opcode of the reference's DAISInterpreter.cc, lookup tables included, bit-exact.  A program is loaded once:
+ * parsed, validated (with the reference's messages, before any device call), compiled into device instructions with
+ * value slots assigned by liveness, and kept resident until da4ml_dais_free.  A lookup index out of range is reported
+ * as the reference reports it with one thread: the first offending sample, then its first offending op. */
+typedef struct da4ml_dais da4ml_dais_t;
+int da4ml_dais_load(const int32_t *program, int64_t n_words, da4ml_dais_t **out);
+/* {n_in, n_out, n_ops, n_tables, value slots L, regime (0 shared memory, 1 global memory), samples per CTA (shared) or
+ * per launch (global), widest dtype in bits} */
+int da4ml_dais_info(const da4ml_dais_t *h, int64_t out[8]);
+/* x [n_samples, n_in], y [n_samples, n_out] float64 in host memory */
+int da4ml_dais_infer(da4ml_dais_t *h, const double *x, int64_t n_samples, double *y);
+/* the same with x and y in device memory (on the device the program was loaded on), on the library's stream */
+int da4ml_dais_infer_device(da4ml_dais_t *h, const double *x_dev, int64_t n_samples, double *y_dev);
+void da4ml_dais_free(da4ml_dais_t *h);
+/* Development switch, read by da4ml_dais_load: shared memory one CTA's slot file may use (a budget below 32 samples'
+ * worth selects the global-memory regime) and samples per launch.  0 = automatic for either. */
+int da4ml_dais_set_shared_budget(int64_t shared_bytes, int64_t chunk_samples);
+
 /* ---- helpers exported by the reference module -------------------------------------------------- */
 /* `csd_decompose` (bindings.cc:63-103 -> bit_decompose.cc:44-62).  csd must hold n_in*n_out*32 int8;
  * *n_bits receives N, the caller reads csd as [n_in, n_out, N].  shift0[n_in], shift1[n_out] int8. */
