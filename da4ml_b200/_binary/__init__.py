@@ -65,6 +65,10 @@ _L.da4ml_dais_infer_device.argtypes = [_vp, _vp, C.c_int64, _vp]
 _L.da4ml_dais_free.argtypes = [_vp]
 _L.da4ml_dais_free.restype = None
 _L.da4ml_dais_set_shared_budget.argtypes = [C.c_int64, C.c_int64]
+_L.da4ml_dais_profile.argtypes = [_vp, _vp, C.c_int64, _i64p, _i64p]
+_L.da4ml_dais_profile_device.argtypes = [_vp, _vp, C.c_int64, _i64p, _i64p]
+_L.da4ml_dais_capture.argtypes = [_vp, _vp, C.c_int64, _i32p, C.c_int32, _vp]
+_L.da4ml_dais_capture_device.argtypes = [_vp, _vp, C.c_int64, _i32p, C.c_int32, _vp]
 _L.da4ml_cmvm_get_lsb_loc.argtypes = [C.c_float]
 _L.da4ml_cmvm_iceil_log2.argtypes = [C.c_float]
 _L.da4ml_cmvm_cost_add.argtypes = [_f32p, _f32p, C.c_int64, C.c_int, C.c_int, C.c_int, _f32p]
@@ -78,7 +82,7 @@ EXPORTED_SYMBOLS = [
     'da4ml_cmvm_csd_decompose', 'da4ml_cmvm_int_arr_to_csd', 'da4ml_cmvm_kernel_decompose',
     'da4ml_cmvm_get_lsb_loc', 'da4ml_cmvm_iceil_log2', 'da4ml_cmvm_cost_add', 'da4ml_dais_run',
     'da4ml_dais_load', 'da4ml_dais_info', 'da4ml_dais_infer', 'da4ml_dais_infer_device', 'da4ml_dais_free',
-    'da4ml_dais_set_shared_budget',
+    'da4ml_dais_set_shared_budget', 'da4ml_dais_profile', 'da4ml_dais_profile_device', 'da4ml_dais_capture', 'da4ml_dais_capture_device',
 ]  # fmt: skip
 
 COUNTER_NAMES = ['status', 'n_ops', 'T', 'sum_F', 'sum_R', 'F0', 'R0', 'D_final', 'F_max', 'compactions', 'D0', 'n_bits', 'group_ctas',

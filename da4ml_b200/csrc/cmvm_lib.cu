@@ -57,18 +57,42 @@ struct da4ml_pipeline {
     std::unique_ptr<PipelineImpl> impl;
 };
 
+// The every-op variant of a program (dais_compile with every_op) on the device: the profile variant is compiled once,
+// lazily, and kept; a capture variant is compiled per call into the same kind of buffer, reused while it is big enough.
+struct DaisVariant {
+    DaisCompiled P;
+    int tile = 0;
+    long long chunk = 0;
+    void *mem = nullptr; // instructions | side table | capture columns | totals [4][n_ops] | first-outside key
+    size_t cap = 0;
+    DaisInstr *d_prog = nullptr;
+    DaisObsEntry *d_obs = nullptr;
+    int32_t *d_cols = nullptr;
+    long long *d_totals = nullptr;
+    unsigned long long *d_first = nullptr;
+    ~DaisVariant() {
+        if (mem)
+            cudaFree(mem);
+    }
+};
+
 // A DAIS program compiled for the device and kept resident (host_dais.cuh, dais_exec.cuh).
 struct da4ml_dais {
     DaisCompiled P;
+    std::vector<int32_t> words; // the program, for the variants
     int device = -1;
     int tile = 0;           // samples per CTA in the shared regime; 0 = global regime
     long long chunk = 0;    // samples per launch
+    long long budget = 0;   // shared memory a CTA's slot file may use, as fixed at load
+    long long forced_chunk = 0;
+    int optin = 0;
     bool has_lookup = false;
     void *mem = nullptr;    // instructions | tables | error word, v0 word
     DaisInstr *d_prog = nullptr;
     int32_t *d_tables = nullptr;
     unsigned long long *d_err = nullptr;
     long long *d_v0 = nullptr;
+    std::unique_ptr<DaisVariant> profile, capture;
     ~da4ml_dais() {
         if (mem)
             cudaFree(mem);
@@ -78,25 +102,38 @@ struct da4ml_dais {
 namespace {
 long long g_dais_shared_budget = 0; // bytes of shared memory for one CTA's slot file; 0 = what the device allows
 long long g_dais_chunk = 0;         // samples per launch; 0 = automatic
-DevBuf g_dais_arena, g_dais_io;
+DevBuf g_dais_arena, g_dais_io, g_dais_rec;
 
-void dais_launch(const da4ml_dais *h, const double *x, double *y, long long n, long long sample0, unsigned long long *err, long long *err_v0) {
-    const DaisCompiled &P = h->P;
+// One compiled stream on the device: predict's, or a variant's.
+struct DaisStream {
+    const DaisCompiled &P;
+    const DaisInstr *prog;
+    int tile;
+    const int32_t *tables;
+};
+DaisStream dais_stream(const da4ml_dais *h) { return {h->P, h->d_prog, h->tile, h->d_tables}; }
+DaisStream dais_stream(const da4ml_dais *h, const DaisVariant &V) { return {V.P, V.d_prog, V.tile, h->d_tables}; }
+
+template <class Obs = DaisNoObserver>
+void dais_launch(const DaisStream &D, const double *x, double *y, long long n, long long sample0, unsigned long long *err, long long *err_v0, Obs obs = Obs()) {
+    const DaisCompiled &P = D.P;
     const int n_instr = (int)P.prog.size();
-    if (h->tile > 0) {
-        const size_t smem = (size_t)8 * std::max(P.n_slots, 1) * h->tile;
-        dais_exec_kernel<true><<<(unsigned)((n + h->tile - 1) / h->tile), h->tile, smem, g_stream>>>(h->d_prog, n_instr, x, P.n_in, y, P.n_out, n, nullptr, 0, h->d_tables, err, sample0, err_v0);
+    if (D.tile > 0) {
+        const size_t smem = (size_t)8 * std::max(P.n_slots, 1) * D.tile;
+        dais_exec_kernel<true, Obs><<<(unsigned)((n + D.tile - 1) / D.tile), D.tile, smem, g_stream>>>(D.prog, n_instr, x, P.n_in, y, P.n_out, n, nullptr, 0, D.tables, err, sample0, err_v0, obs);
     }
     else {
-        g_dais_arena.ensure((size_t)8 * std::max(P.n_slots, 1) * std::max(n, 1LL), false);
-        dais_exec_kernel<false><<<(unsigned)((n + 255) / 256), 256, 0, g_stream>>>(h->d_prog, n_instr, x, P.n_in, y, P.n_out, n, (long long *)g_dais_arena.p, n, h->d_tables, err, sample0, err_v0);
+        // an observer runs whole warps, so the lanes past n need arena columns too
+        const long long stride = Obs::kActive ? (n + 255) / 256 * 256 : n;
+        g_dais_arena.ensure((size_t)8 * std::max(P.n_slots, 1) * std::max(stride, 1LL), false);
+        dais_exec_kernel<false, Obs><<<(unsigned)((n + 255) / 256), 256, 0, g_stream>>>(D.prog, n_instr, x, P.n_in, y, P.n_out, n, (long long *)g_dais_arena.p, stride, D.tables, err, sample0, err_v0, obs);
     }
     CK(cudaGetLastError());
 }
 
 // After the launches of a call: raise the reference's message for the first (sample, op) whose lookup was out of range.
 // That sample is run once more on its own to recover the operand.  `row(s)` is a device pointer to input row s.
-template <class Row> void dais_check(const da4ml_dais *h, Row row, double *y_scratch) {
+template <class Row> void dais_check(const da4ml_dais *h, const DaisStream &D, Row row, double *y_scratch) {
     if (!h->has_lookup)
         return;
     unsigned long long key = 0;
@@ -104,14 +141,133 @@ template <class Row> void dais_check(const da4ml_dais *h, Row row, double *y_scr
     CK(cudaStreamSynchronize(g_stream));
     if (key == ~0ull)
         return;
-    const unsigned long long n_instr = h->P.prog.size();
+    const unsigned long long n_instr = D.P.prog.size();
     const long long s = (long long)(key / n_instr);
     const int pc = (int)(key % n_instr);
-    dais_launch(h, row(s), y_scratch, 1, 0, h->d_err + 1, h->d_v0);
+    dais_launch(D, row(s), y_scratch, 1, 0, h->d_err + 1, h->d_v0);
     long long v0 = 0;
     CK(cudaMemcpyAsync(&v0, h->d_v0, sizeof(v0), cudaMemcpyDeviceToHost, g_stream));
     CK(cudaStreamSynchronize(g_stream));
-    throw ApiError(DA4ML_E_RUNTIME, dais_lookup_message(h->P, pc, v0));
+    throw ApiError(DA4ML_E_RUNTIME, dais_lookup_message(D.P, pc, v0));
+}
+
+// Compiles the every-op variant of h's program into V (capturing ops[0..k), if any) and uploads it; V's buffer is
+// reused while it is big enough.  A profile's launches are sized so that the per-warp records stay within 1 GB.
+void dais_variant_build(const da4ml_dais *h, DaisVariant &V, const int32_t *ops, int k, bool profile) {
+    try {
+        V.P = dais_compile(h->words.data(), (long long)h->words.size(), true, ops, k);
+    }
+    catch (const std::runtime_error &e) {
+        throw ApiError(DA4ML_E_INVALID, e.what());
+    }
+    const DaisCompiled &P = V.P;
+    V.tile = dais_shared_tile(P.n_slots, h->budget);
+    if (V.tile > 0) {
+        V.chunk = 1LL << 24;
+        CK(cudaFuncSetAttribute(dais_exec_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->optin));
+        CK(cudaFuncSetAttribute(dais_exec_kernel<true, DaisProfileObserver>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->optin));
+        CK(cudaFuncSetAttribute(dais_exec_kernel<true, DaisCaptureObserver>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->optin));
+    }
+    else
+        V.chunk = std::max<long long>(256, ((1LL << 31) / (8LL * std::max(P.n_slots, 1))) / 256 * 256);
+    V.chunk = std::min<long long>(V.chunk, std::max<long long>(256, ((1LL << 28) / (8LL * std::max(1, P.n_in + k))) / 256 * 256));
+    if (profile)
+        V.chunk = dais_profile_chunk((long long)P.prog.size(), V.chunk, 1LL << 30);
+    if (h->forced_chunk > 0)
+        V.chunk = h->forced_chunk;
+    Carver c;
+    const size_t o_prog = c.take(sizeof(DaisInstr) * P.prog.size()), o_obs = c.take(sizeof(DaisObsEntry) * P.obs.size()), o_cols = c.take(sizeof(int32_t) * P.cap_cols.size()),
+                 o_tot = c.take(sizeof(long long) * (4 * (size_t)P.n_ops + 1));
+    if (c.off > V.cap) {
+        if (V.mem)
+            CK(cudaFree(V.mem));
+        V.mem = nullptr;
+        V.cap = 0;
+        CK(cudaMalloc(&V.mem, c.off));
+        V.cap = c.off;
+    }
+    char *b = (char *)V.mem;
+    V.d_prog = (DaisInstr *)(b + o_prog);
+    V.d_obs = (DaisObsEntry *)(b + o_obs);
+    V.d_cols = (int32_t *)(b + o_cols);
+    V.d_totals = (long long *)(b + o_tot);
+    V.d_first = (unsigned long long *)(V.d_totals + 4 * (size_t)P.n_ops);
+    if (!P.prog.empty()) {
+        CK(cudaMemcpyAsync(V.d_prog, P.prog.data(), sizeof(DaisInstr) * P.prog.size(), cudaMemcpyHostToDevice, g_stream));
+        CK(cudaMemcpyAsync(V.d_obs, P.obs.data(), sizeof(DaisObsEntry) * P.obs.size(), cudaMemcpyHostToDevice, g_stream));
+    }
+    if (!P.cap_cols.empty())
+        CK(cudaMemcpyAsync(V.d_cols, P.cap_cols.data(), sizeof(int32_t) * P.cap_cols.size(), cudaMemcpyHostToDevice, g_stream));
+}
+
+// The profile of n > 0 samples into stats [4][n_ops] (min, max, outside, wrapped) and first {sample, op}.
+// `stage(s0, m)` gives a device pointer to input rows [s0, s0 + m), valid until the next call; `row(s)` one row.
+// Totals stay on the device across the launches and come back once.
+template <class Stage, class Row> void dais_profile_run(da4ml_dais *h, long long n, Stage stage, Row row, int64_t *stats, int64_t *first) {
+    if (!h->profile) {
+        auto V = std::make_unique<DaisVariant>();
+        dais_variant_build(h, *V, nullptr, 0, true);
+        h->profile = std::move(V);
+    }
+    const DaisVariant &V = *h->profile;
+    const DaisCompiled &P = V.P;
+    const DaisStream D = dais_stream(h, V);
+    const int n_instr = (int)P.prog.size();
+    const size_t n_tot = 4 * (size_t)P.n_ops + 1;
+    std::vector<long long> tot(n_tot, 0);
+    std::fill(tot.begin(), tot.begin() + P.n_ops, (long long)0x7fffffffffffffffll);
+    std::fill(tot.begin() + P.n_ops, tot.begin() + 2 * P.n_ops, (long long)0x8000000000000000ull);
+    tot[n_tot - 1] = -1;
+    CK(cudaMemcpyAsync(V.d_totals, tot.data(), sizeof(long long) * n_tot, cudaMemcpyHostToDevice, g_stream));
+    CK(cudaMemsetAsync(h->d_err, 0xff, 2 * sizeof(unsigned long long), g_stream));
+    const long long C = std::min<long long>(V.chunk, n);
+    g_dais_rec.ensure((size_t)32 * std::max(n_instr, 1) * ((C + 31) / 32), false);
+    for (long long s0 = 0; s0 < n; s0 += C) {
+        const long long Sc = std::min<long long>(C, n - s0);
+        const double *xs = stage(s0, Sc);
+        DaisProfileObserver obs{};
+        obs.side = V.d_obs, obs.rec = (long long *)g_dais_rec.p, obs.n_warps = (Sc + 31) / 32, obs.first = V.d_first, obs.n_ops = P.n_ops;
+        dais_launch(D, xs, nullptr, Sc, s0, h->d_err, nullptr, obs);
+        if (n_instr > 0) {
+            dais_profile_merge_kernel<<<(unsigned)(((long long)n_instr * 32 + 255) / 256), 256, 0, g_stream>>>(obs.rec, n_instr, obs.n_warps, V.d_obs, V.d_totals, P.n_ops);
+            CK(cudaGetLastError());
+        }
+        dais_check(h, D, row, nullptr);
+    }
+    CK(cudaMemcpyAsync(tot.data(), V.d_totals, sizeof(long long) * n_tot, cudaMemcpyDeviceToHost, g_stream));
+    CK(cudaStreamSynchronize(g_stream));
+    std::copy(tot.begin(), tot.end() - 1, stats);
+    const unsigned long long key = (unsigned long long)tot[n_tot - 1];
+    first[0] = key == ~0ull ? -1 : (int64_t)(key / (unsigned long long)P.n_ops);
+    first[1] = key == ~0ull ? -1 : (int64_t)(key % (unsigned long long)P.n_ops);
+}
+
+// The values of ops[0..k) for n > 0 samples: `stage` / `row` as above; `dst(s0, m)` gives the device rows [s0, s0 + m)
+// of the [n][k] int64 result, and `flush(s0, m)` is called once they are written.
+template <class Stage, class Row, class Dst, class Flush>
+void dais_capture_run(da4ml_dais *h, long long n, const int32_t *ops, int k, Stage stage, Row row, Dst dst, Flush flush) {
+    if (!h->capture)
+        h->capture = std::make_unique<DaisVariant>();
+    DaisVariant &V = *h->capture;
+    dais_variant_build(h, V, ops, k, false);
+    const DaisStream D = dais_stream(h, V);
+    CK(cudaMemsetAsync(h->d_err, 0xff, 2 * sizeof(unsigned long long), g_stream));
+    for (long long s0 = 0; s0 < n; s0 += V.chunk) {
+        const long long Sc = std::min<long long>(V.chunk, n - s0);
+        const double *xs = stage(s0, Sc); // (before dst: the host path carves both from one staging buffer)
+        DaisCaptureObserver obs{};
+        obs.side = V.d_obs, obs.cols = V.d_cols, obs.out = dst(s0, Sc), obs.k = k;
+        dais_launch(D, xs, nullptr, Sc, s0, h->d_err, nullptr, obs);
+        dais_check(h, D, row, nullptr);
+        flush(s0, Sc);
+    }
+}
+
+// The op list of a capture call, checked before any device call.
+void dais_check_ops(const da4ml_dais *h, const int32_t *ops, int k) {
+    for (int j = 0; j < k; ++j)
+        if (ops[j] < 0 || ops[j] >= h->P.n_ops)
+            throw ApiError(DA4ML_E_INVALID, "op index " + std::to_string(ops[j]) + " out of range [0, " + std::to_string(h->P.n_ops) + ")");
 }
 
 void dais_check_device(const da4ml_dais *h) {
@@ -620,12 +776,16 @@ int da4ml_dais_load(const int32_t *program, int64_t n_words, da4ml_dais_t **out)
         }
         init_device();
         h->device = g_device;
+        h->words.assign(program, program + n_words);
         const DaisCompiled &P = h->P;
         for (const DaisInstr &I : P.prog)
             h->has_lookup |= I.kind == DK_LOOKUP;
         int optin = 0;
         CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, g_device));
         const long long budget = g_dais_shared_budget > 0 ? std::min<long long>(g_dais_shared_budget, optin) : optin;
+        h->budget = budget;
+        h->forced_chunk = g_dais_chunk;
+        h->optin = optin;
         h->tile = dais_shared_tile(P.n_slots, budget);
         if (h->tile > 0) {
             CK(cudaFuncSetAttribute(dais_exec_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
@@ -685,8 +845,8 @@ int da4ml_dais_infer(da4ml_dais_t *h, const double *x, int64_t n_samples, double
             const long long Sc = std::min<long long>(C, n_samples - s0);
             if (P.n_in)
                 CK(cudaMemcpyAsync(dx, x + s0 * P.n_in, sizeof(double) * Sc * P.n_in, cudaMemcpyHostToDevice, g_stream));
-            dais_launch(h, dx, dy, Sc, s0, h->d_err, nullptr);
-            dais_check(h, [&](long long s) {
+            dais_launch(dais_stream(h), dx, dy, Sc, s0, h->d_err, nullptr);
+            dais_check(h, dais_stream(h), [&](long long s) {
                 CK(cudaMemcpyAsync(dx, x + s * P.n_in, sizeof(double) * P.n_in, cudaMemcpyHostToDevice, g_stream));
                 return (const double *)dx;
             }, dy);
@@ -710,9 +870,103 @@ int da4ml_dais_infer_device(da4ml_dais_t *h, const double *x_dev, int64_t n_samp
         CK(cudaMemsetAsync(h->d_err, 0xff, 2 * sizeof(unsigned long long), g_stream));
         for (long long s0 = 0; s0 < n_samples; s0 += h->chunk) {
             const long long Sc = std::min<long long>(h->chunk, n_samples - s0);
-            dais_launch(h, x_dev + s0 * P.n_in, y_dev + s0 * P.n_out, Sc, s0, h->d_err, nullptr);
+            dais_launch(dais_stream(h), x_dev + s0 * P.n_in, y_dev + s0 * P.n_out, Sc, s0, h->d_err, nullptr);
         }
-        dais_check(h, [&](long long s) { return x_dev + s * P.n_in; }, (double *)g_dais_io.p);
+        dais_check(h, dais_stream(h), [&](long long s) { return x_dev + s * P.n_in; }, (double *)g_dais_io.p);
+    });
+}
+
+namespace {
+void dais_profile_args(const da4ml_dais *h, const double *x, int64_t n_samples, int64_t *stats, int64_t *first) {
+    if (!h || n_samples < 0 || !stats || !first || (n_samples > 0 && !x && h->P.n_in))
+        throw ApiError(DA4ML_E_INVALID, "invalid argument");
+    const int n_ops = h->P.n_ops;
+    std::fill(stats, stats + n_ops, (int64_t)0x7fffffffffffffffll);
+    std::fill(stats + n_ops, stats + 2LL * n_ops, (int64_t)0x8000000000000000ull);
+    std::fill(stats + 2LL * n_ops, stats + 4LL * n_ops, (int64_t)0);
+    first[0] = first[1] = -1;
+}
+void dais_capture_args(const da4ml_dais *h, const double *x, int64_t n_samples, const int32_t *ops, int32_t k, int64_t *out) {
+    if (!h || n_samples < 0 || k < 0 || (k > 0 && !ops) || (n_samples > 0 && ((!x && h->P.n_in) || (!out && k))))
+        throw ApiError(DA4ML_E_INVALID, "invalid argument");
+    dais_check_ops(h, ops, k);
+}
+} // namespace
+
+int da4ml_dais_profile(da4ml_dais_t *h, const double *x, int64_t n_samples, int64_t *stats, int64_t first[2]) {
+    return guarded([&] {
+        dais_profile_args(h, x, n_samples, stats, first);
+        if (n_samples == 0)
+            return;
+        init_device();
+        dais_check_device(h);
+        const int n_in = h->P.n_in;
+        double *dx = nullptr;
+        dais_profile_run(h, n_samples, [&](long long s0, long long m) {
+            g_dais_io.ensure(sizeof(double) * std::max<long long>(m * n_in, 1), false);
+            dx = (double *)g_dais_io.p;
+            if (n_in)
+                CK(cudaMemcpyAsync(dx, x + s0 * n_in, sizeof(double) * m * n_in, cudaMemcpyHostToDevice, g_stream));
+            return (const double *)dx;
+        }, [&](long long s) {
+            CK(cudaMemcpyAsync(dx, x + s * n_in, sizeof(double) * n_in, cudaMemcpyHostToDevice, g_stream));
+            return (const double *)dx;
+        }, stats, first);
+    });
+}
+
+int da4ml_dais_profile_device(da4ml_dais_t *h, const double *x_dev, int64_t n_samples, int64_t *stats, int64_t first[2]) {
+    return guarded([&] {
+        dais_profile_args(h, x_dev, n_samples, stats, first);
+        if (n_samples == 0)
+            return;
+        init_device();
+        dais_check_device(h);
+        const int n_in = h->P.n_in;
+        dais_profile_run(h, n_samples, [&](long long s0, long long) { return x_dev + s0 * n_in; }, [&](long long s) { return x_dev + s * n_in; }, stats, first);
+    });
+}
+
+int da4ml_dais_capture(da4ml_dais_t *h, const double *x, int64_t n_samples, const int32_t *ops, int32_t k, int64_t *out) {
+    return guarded([&] {
+        dais_capture_args(h, x, n_samples, ops, k, out);
+        if (n_samples == 0)
+            return;
+        init_device();
+        dais_check_device(h);
+        const int n_in = h->P.n_in;
+        double *dx = nullptr;
+        long long *dout = nullptr;
+        dais_capture_run(h, n_samples, ops, k, [&](long long s0, long long m) {
+            Carver c;
+            const size_t o_x = c.take(sizeof(double) * std::max<long long>(m * n_in, 1)), o_out = c.take(sizeof(long long) * std::max<long long>(m * k, 1));
+            g_dais_io.ensure(c.off, false);
+            dx = (double *)((char *)g_dais_io.p + o_x);
+            dout = (long long *)((char *)g_dais_io.p + o_out);
+            if (n_in)
+                CK(cudaMemcpyAsync(dx, x + s0 * n_in, sizeof(double) * m * n_in, cudaMemcpyHostToDevice, g_stream));
+            return (const double *)dx;
+        }, [&](long long s) {
+            CK(cudaMemcpyAsync(dx, x + s * n_in, sizeof(double) * n_in, cudaMemcpyHostToDevice, g_stream));
+            return (const double *)dx;
+        }, [&](long long, long long) { return dout; }, [&](long long s0, long long m) {
+            if (k)
+                CK(cudaMemcpyAsync(out + s0 * k, dout, sizeof(long long) * m * k, cudaMemcpyDeviceToHost, g_stream));
+            CK(cudaStreamSynchronize(g_stream));
+        });
+    });
+}
+
+int da4ml_dais_capture_device(da4ml_dais_t *h, const double *x_dev, int64_t n_samples, const int32_t *ops, int32_t k, int64_t *out_dev) {
+    return guarded([&] {
+        dais_capture_args(h, x_dev, n_samples, ops, k, out_dev);
+        if (n_samples == 0)
+            return;
+        init_device();
+        dais_check_device(h);
+        const int n_in = h->P.n_in;
+        dais_capture_run(h, n_samples, ops, k, [&](long long s0, long long) { return x_dev + s0 * n_in; }, [&](long long s) { return x_dev + s * n_in; },
+                         [&](long long s0, long long) { return (long long *)out_dev + s0 * k; }, [](long long, long long) {});
     });
 }
 

@@ -16,6 +16,18 @@
 #ifndef DA_CPU_SIM
 #include <cuda_runtime.h>
 #define DA_DYN_SHARED(name) extern __shared__ __align__(16) unsigned char name[]
+#else
+// the CPU simulation of the kernels (tests/simt) has no redux.sync: the same 32-bit warp reductions on its shuffles
+template <class T, class F> T da_sim_reduce(unsigned m, T v, F f) {
+    for (int o = 16; o > 0; o >>= 1)
+        v = f(v, __shfl_xor_sync(m, v, o));
+    return v;
+}
+inline int __reduce_min_sync(unsigned m, int v) { return da_sim_reduce(m, v, [](int a, int b) { return a < b ? a : b; }); }
+inline unsigned __reduce_min_sync(unsigned m, unsigned v) { return da_sim_reduce(m, v, [](unsigned a, unsigned b) { return a < b ? a : b; }); }
+inline int __reduce_max_sync(unsigned m, int v) { return da_sim_reduce(m, v, [](int a, int b) { return a > b ? a : b; }); }
+inline unsigned __reduce_max_sync(unsigned m, unsigned v) { return da_sim_reduce(m, v, [](unsigned a, unsigned b) { return a > b ? a : b; }); }
+inline unsigned __reduce_add_sync(unsigned m, unsigned v) { return da_sim_reduce(m, v, [](unsigned a, unsigned b) { return a + b; }); }
 #endif
 
 namespace da {
@@ -84,17 +96,40 @@ __device__ __forceinline__ long long dx_f2i(double f) {
     return (long long)f;
 }
 
+// Per-instruction side table of the profile / capture variants (host_dais.cuh, dais_compile_variant), read only by the
+// observers below; the instruction stream itself is the one predict runs.
+//   op         the op this instruction computes
+//   cap_begin  its capture columns are cols[cap_begin .. cap_begin + cap_count) (duplicates in the request included)
+//   quant      1 for the ops whose value passes a wrap step (-1, +-2, +-3, +-6)
+//   lo, hi     the declared dtype's range, folded on the host
+struct DaisObsEntry {
+    int32_t op, cap_begin, cap_count, quant;
+    long long lo, hi;
+};
+static_assert(sizeof(DaisObsEntry) == 32, "DaisObsEntry is 32 bytes");
+
+// The observer of predict: sees nothing, costs nothing.
+struct DaisNoObserver {
+    static constexpr bool kActive = false;
+    __device__ __forceinline__ void begin(long long, long long, bool) {}
+    __device__ __forceinline__ void operator()(int, long long, long long) {}
+    __device__ __forceinline__ void end() {}
+};
+
 // Runs the compiled program for one sample.  `S(k)` is a reference to the sample's slot k.  Returns the index of the
 // first instruction whose table index was out of range (its result is 0), or -1; `*err_v0` receives that operand.
-template <class Slots>
-__device__ __forceinline__ int dais_exec_sample(const DaisInstr *__restrict__ prog, int n_instr, const double *__restrict__ x, double *__restrict__ y, const int32_t *__restrict__ tables, Slots S, long long *err_v0) {
+// `obs(pc, r, pre)` sees every result r; for the kinds with a wrap step, `pre` is the value before it (the converted
+// input, the shifted operand; equal to r where relu clamps a negative operand to 0).
+template <class Slots, class Obs>
+__device__ __forceinline__ int dais_exec_sample(const DaisInstr *__restrict__ prog, int n_instr, const double *__restrict__ x, double *__restrict__ y, const int32_t *__restrict__ tables, Slots S, long long *err_v0, Obs &obs) {
     int first_err = -1;
     for (int pc = 0; pc < n_instr; ++pc) {
         const DaisInstr I = prog[pc];
-        long long r = 0;
+        long long r = 0, pre = 0;
         switch (I.kind) {
         case DK_INPUT:
-            r = dx_wrap(dx_f2i(floor(x[I.a] * dx_bits_to_double(I.k2))), I.k0, I.k1, I.aux1 != 0);
+            pre = dx_f2i(floor(x[I.a] * dx_bits_to_double(I.k2)));
+            r = dx_wrap(pre, I.k0, I.k1, I.aux1 != 0);
             break;
         case DK_SHIFT_ADD: {
             const long long v1 = S(I.a);
@@ -108,6 +143,7 @@ __device__ __forceinline__ int dais_exec_sample(const DaisInstr *__restrict__ pr
         case DK_QUANT: {
             const long long v = I.neg ? dx_neg(S(I.a)) : S(I.a);
             r = (I.kind == DK_RELU && v < 0) ? 0 : dx_wrap(dx_sar(v, I.s0), I.k0, I.k1, I.aux1 != 0);
+            pre = (I.kind == DK_RELU && v < 0) ? 0 : dx_sar(v, I.s0);
             break;
         }
         case DK_CONST_ADD:
@@ -119,8 +155,8 @@ __device__ __forceinline__ int dais_exec_sample(const DaisInstr *__restrict__ pr
         case DK_MUX: {
             const long long vc = S(I.c);
             const bool cond = I.aux0 ? vc < 0 : vc > I.k2;
-            r = cond ? dx_shl(S(I.a), I.s0) : dx_shl(I.neg ? dx_neg(S(I.b)) : S(I.b), I.s1);
-            r = dx_wrap(r, I.k0, I.k1, I.aux1 != 0);
+            pre = cond ? dx_shl(S(I.a), I.s0) : dx_shl(I.neg ? dx_neg(S(I.b)) : S(I.b), I.s1);
+            r = dx_wrap(pre, I.k0, I.k1, I.aux1 != 0);
             break;
         }
         case DK_MUL:
@@ -169,6 +205,7 @@ __device__ __forceinline__ int dais_exec_sample(const DaisInstr *__restrict__ pr
             continue;
         }
         S(I.dst) = r;
+        obs(pc, r, pre);
     }
     return first_err;
 }
@@ -181,27 +218,146 @@ __device__ __forceinline__ void dais_report(unsigned long long *err, long long s
         atomicMin(err, (unsigned long long)sample * (unsigned long long)n_instr + (unsigned long long)pc);
 }
 
+// 64-bit warp minimum / maximum on the 32-bit reduction unit: the extreme high word first, then the extreme low word
+// among the lanes that hold it.  Every lane gets the result.
+__device__ __forceinline__ long long dx_warp_min(long long v) {
+    const int hi = (int)(v >> 32);
+    const int mh = __reduce_min_sync(0xffffffffu, hi);
+    const unsigned ml = __reduce_min_sync(0xffffffffu, hi == mh ? (unsigned)v : 0xffffffffu);
+    return (long long)(((unsigned long long)(unsigned)mh << 32) | ml);
+}
+__device__ __forceinline__ long long dx_warp_max(long long v) {
+    const int hi = (int)(v >> 32);
+    const int mh = __reduce_max_sync(0xffffffffu, hi);
+    const unsigned ml = __reduce_max_sync(0xffffffffu, hi == mh ? (unsigned)v : 0u);
+    return (long long)(((unsigned long long)(unsigned)mh << 32) | ml);
+}
+
+// Profile observer: per instruction, one warp's samples reduced to a 32-byte record {min, max, outside, wrapped} in
+// rec[pc][warp] (`n_warps` warps in this launch), merged per op afterwards by dais_profile_merge_kernel.  Dispatch is
+// warp-uniform, so every lane of a warp reaches every reduction; lanes past the launch's samples contribute nothing.
+// The first value outside its range is kept per warp as the key sample * n_ops + op (sample order first, then op
+// order) and folded into `*first` with one atomicMin when the warp is done.
+struct DaisProfileObserver {
+    static constexpr bool kActive = true;
+    const DaisObsEntry *__restrict__ side;
+    long long *__restrict__ rec;
+    long long n_warps;
+    unsigned long long *first;
+    long long n_ops;
+    // this thread
+    long long warp, sample; // warp index in the launch; sample (in the whole call) of the warp's lane 0
+    int lane;
+    bool valid;
+    unsigned long long key;
+
+    __device__ __forceinline__ void begin(long long sample0, long long s, bool v) {
+        lane = (int)(s & 31);
+        warp = s >> 5;
+        sample = sample0 + (s - lane);
+        valid = v;
+        key = ~0ull;
+    }
+    __device__ __forceinline__ void operator()(int pc, long long r, long long pre) {
+        const DaisObsEntry e = side[pc];
+        const long long mn = dx_warp_min(valid ? r : (long long)0x7fffffffffffffffll);
+        const long long mx = dx_warp_max(valid ? r : (long long)0x8000000000000000ull);
+        const unsigned out = __ballot_sync(0xffffffffu, valid && (r < e.lo || r > e.hi));
+        const unsigned wr = e.quant ? __ballot_sync(0xffffffffu, valid && pre != r) : 0u;
+        if (out) {
+            const unsigned long long k = (unsigned long long)(sample + __ffs((int)out) - 1) * (unsigned long long)n_ops + (unsigned long long)e.op;
+            key = k < key ? k : key;
+        }
+        if (lane < 4)
+            rec[((long long)pc * n_warps + warp) * 4 + lane] = lane == 0 ? mn : lane == 1 ? mx : lane == 2 ? (long long)__popc(out) : (long long)__popc(wr);
+    }
+    __device__ __forceinline__ void end() {
+        if (lane == 0 && key != ~0ull)
+            atomicMin(first, key);
+    }
+};
+
+// Capture observer: the values of the ops marked in the side table, written through to out[s][col] when they run.
+struct DaisCaptureObserver {
+    static constexpr bool kActive = true;
+    const DaisObsEntry *__restrict__ side;
+    const int32_t *__restrict__ cols;
+    long long *__restrict__ out; // [n][k] of this launch
+    int k;
+    long long *row;
+
+    __device__ __forceinline__ void begin(long long, long long s, bool v) { row = v ? out + s * k : nullptr; }
+    __device__ __forceinline__ void operator()(int pc, long long r, long long) {
+        if (!row)
+            return;
+        const DaisObsEntry e = side[pc];
+        for (int j = 0; j < e.cap_count; ++j)
+            row[cols[e.cap_begin + j]] = r;
+    }
+    __device__ __forceinline__ void end() {}
+};
+
 // SHARED: the CTA's slot file is [L][blockDim.x] int64 in dynamic shared memory.  Otherwise slot k of sample s is
 // arena[k * stride + s] (s counted within this launch).  x / y: [n][n_in] / [n][n_out] of this launch; `sample0` is the
 // index of its first sample in the whole call (error keys only).
-template <bool SHARED>
+// With an active observer every warp that holds a sample of the launch runs whole (its reductions are full-mask
+// collectives): the lanes past n run the last sample, write nothing and report no lookup error.  The arena then needs
+// stride >= the launch's threads.
+template <bool SHARED, class Obs = DaisNoObserver>
 __global__ void __launch_bounds__(256) dais_exec_kernel(const DaisInstr *__restrict__ prog, int n_instr, const double *__restrict__ x, int n_in, double *__restrict__ y, int n_out, long long n,
-                                                        long long *__restrict__ arena, long long stride, const int32_t *__restrict__ tables, unsigned long long *err, long long sample0, long long *err_v0) {
+                                                        long long *__restrict__ arena, long long stride, const int32_t *__restrict__ tables, unsigned long long *err, long long sample0, long long *err_v0,
+                                                        Obs obs = Obs()) {
     const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (s >= n)
+    if (Obs::kActive ? (s & ~31LL) >= n : s >= n)
         return;
+    const bool valid = s < n;
+    const long long sx = valid ? s : n - 1;
+    Obs o = obs; // (a register copy: a reference to the parameter itself would put it in local memory)
+    o.begin(sample0, s, valid);
     int pc;
     if (SHARED) {
         DA_DYN_SHARED(dais_smem);
         long long *base = reinterpret_cast<long long *>(dais_smem) + threadIdx.x;
         const int T = (int)blockDim.x;
-        pc = dais_exec_sample(prog, n_instr, x + s * n_in, y + s * n_out, tables, [=](int k) -> long long & { return base[(long long)k * T]; }, err_v0);
+        pc = dais_exec_sample(prog, n_instr, x + sx * n_in, y + sx * n_out, tables, [=](int k) -> long long & { return base[(long long)k * T]; }, err_v0, o);
     }
     else {
         long long *base = arena + s;
-        pc = dais_exec_sample(prog, n_instr, x + s * n_in, y + s * n_out, tables, [=](int k) -> long long & { return base[(long long)k * stride]; }, err_v0);
+        pc = dais_exec_sample(prog, n_instr, x + sx * n_in, y + sx * n_out, tables, [=](int k) -> long long & { return base[(long long)k * stride]; }, err_v0, o);
     }
-    dais_report(err, sample0 + s, n_instr, pc);
+    o.end();
+    if (valid)
+        dais_report(err, sample0 + s, n_instr, pc);
+}
+
+// Folds the records of one profile launch (rec[n_instr][n_warps][4]) into the per-op totals [4][n_ops]: min, max,
+// outside, wrapped.  One warp per instruction; each op has exactly one instruction in the profile variant, so no two
+// warps touch the same total, and launches on one stream follow each other.
+__global__ void __launch_bounds__(256) dais_profile_merge_kernel(const long long *__restrict__ rec, int n_instr, long long n_warps, const DaisObsEntry *__restrict__ side, long long *__restrict__ totals, int n_ops) {
+    const int pc = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    const int lane = (int)(threadIdx.x & 31);
+    if (pc >= n_instr)
+        return;
+    long long mn = 0x7fffffffffffffffll, mx = (long long)0x8000000000000000ull;
+    unsigned out = 0, wr = 0; // at most one launch's samples
+    for (long long w = lane; w < n_warps; w += 32) {
+        const long long *r = rec + ((long long)pc * n_warps + w) * 4;
+        mn = r[0] < mn ? r[0] : mn;
+        mx = r[1] > mx ? r[1] : mx;
+        out += (unsigned)r[2];
+        wr += (unsigned)r[3];
+    }
+    mn = dx_warp_min(mn);
+    mx = dx_warp_max(mx);
+    out = __reduce_add_sync(0xffffffffu, out);
+    wr = __reduce_add_sync(0xffffffffu, wr);
+    if (lane == 0) {
+        long long *t = totals + side[pc].op;
+        t[0] = mn < t[0] ? mn : t[0];
+        t[n_ops] = mx > t[n_ops] ? mx : t[n_ops];
+        t[2LL * n_ops] += out;
+        t[3LL * n_ops] += wr;
+    }
 }
 
 } // namespace da

@@ -26,6 +26,9 @@ struct DaisCompiled {
     std::vector<int> op_slot;     // slot of op i, -1 for an op whose value nobody reads (not compiled)
     std::vector<int> instr_op;    // op of each instruction (-1 for outputs)
     std::vector<int32_t> table_size;
+    // profile / capture variants only (dais_compile with every_op): one entry per instruction, and the capture columns
+    std::vector<DaisObsEntry> obs;
+    std::vector<int32_t> cap_cols;
 };
 
 namespace dais_detail {
@@ -46,10 +49,35 @@ struct Op {
 inline std::string s(long long v) { return std::to_string(v); }
 inline bool reads_id0(int opc) { return opc != -1 && opc != 5; }
 inline bool reads_id1(int opc) { return opc == 0 || opc == 1 || opc == 6 || opc == -6 || opc == 7 || opc == 10; }
+inline bool wraps(int opc) { return opc == -1 || std::abs(opc) == 2 || std::abs(opc) == 3 || std::abs(opc) == 6; }
 } // namespace dais_detail
 
+// The range of a declared dtype, with w = is_signed + integers + fractionals in 64-bit (not the reference's int32):
+// w <= 0 holds only 0; 1 <= w <= 63 the usual two's-complement or unsigned range; w >= 64 is unbounded (unsigned: >= 0).
+inline void dais_dtype_range(int32_t is_signed, int32_t integers, int32_t fractionals, long long &lo, long long &hi) {
+    const long long w = (is_signed ? 1LL : 0LL) + integers + fractionals;
+    if (w <= 0)
+        lo = hi = 0;
+    else if (w >= 64) {
+        lo = is_signed ? (long long)0x8000000000000000ull : 0;
+        hi = 0x7fffffffffffffffll;
+    }
+    else if (is_signed) {
+        lo = -(1LL << (w - 1));
+        hi = (1LL << (w - 1)) - 1;
+    }
+    else {
+        lo = 0;
+        hi = (long long)((1ull << w) - 1);
+    }
+}
+
 // Parse, validate and compile.  Throws std::runtime_error with the reference's message where it has one.
-inline DaisCompiled dais_compile(const int32_t *w, long long n_words) {
+// `every_op` compiles the profile / capture variant: every op runs, as in the reference (none is skipped for want of
+// a reader), no output instructions are emitted, and each instruction gets a side-table entry (P.obs).  The ops listed
+// in `capture` (duplicates allowed) are marked for the capture observer, column j for capture[j]; like outputs, they
+// are written through when they run and do not lengthen any slot's lifetime.
+inline DaisCompiled dais_compile(const int32_t *w, long long n_words, bool every_op = false, const int32_t *capture = nullptr, int n_capture = 0) {
     using namespace dais_detail;
     if (!w || n_words < 6)
         throw std::runtime_error("Binary data too small to contain valid DAIS model file");
@@ -121,6 +149,14 @@ inline DaisCompiled dais_compile(const int32_t *w, long long n_words) {
     for (int o = 0; o < P.n_out; ++o)
         if (out_idxs[o] < -1 || out_idxs[o] >= n)
             throw std::runtime_error("output index out of range at output " + s(o));
+    if (n_capture > 0 && !every_op)
+        throw std::logic_error("ops are captured by the every-op variant only");
+    std::vector<std::vector<int>> cols_of(every_op ? n : 0);
+    for (int j = 0; j < n_capture; ++j) {
+        if (capture[j] < 0 || capture[j] >= n)
+            throw std::runtime_error("op index " + s(capture[j]) + " out of range [0, " + s(n) + ")");
+        cols_of[capture[j]].push_back(j);
+    }
 
     // liveness: last reader of every value; outputs are written through when their op runs and do not extend it
     std::vector<int> last_use(n, -1);
@@ -148,7 +184,7 @@ inline DaisCompiled dais_compile(const int32_t *w, long long n_words) {
             last_use[v] = -2; // (an op may read one value twice)
         }
     };
-    for (int o = 0; o < P.n_out; ++o)
+    for (int o = 0; o < P.n_out && !every_op; ++o)
         if (out_idxs[o] < 0) {
             DaisInstr I{};
             I.kind = DK_OUTPUT, I.dst = o, I.a = -1;
@@ -159,7 +195,7 @@ inline DaisCompiled dais_compile(const int32_t *w, long long n_words) {
         const Op &op = ops[i];
         const int opc = op.opcode;
         // a value nobody reads is not computed; a lookup still is (its index check is observable)
-        if (last_use[i] < 0 && !is_out[i] && opc != 8)
+        if (!every_op && last_use[i] < 0 && !is_out[i] && opc != 8)
             continue;
         DaisInstr I{};
         auto slot = [&](int v) { return P.op_slot[v]; };
@@ -253,6 +289,16 @@ inline DaisCompiled dais_compile(const int32_t *w, long long n_words) {
         free_slots.pop_back();
         P.prog.push_back(I);
         P.instr_op.push_back(i);
+        if (every_op) {
+            DaisObsEntry E{};
+            E.op = i, E.cap_begin = (int32_t)P.cap_cols.size(), E.cap_count = (int32_t)cols_of[i].size(), E.quant = wraps(opc) ? 1 : 0;
+            dais_dtype_range(op.is_signed, op.integers, op.fractionals, E.lo, E.hi);
+            P.obs.push_back(E);
+            P.cap_cols.insert(P.cap_cols.end(), cols_of[i].begin(), cols_of[i].end());
+            if (last_use[i] < 0)
+                free_slots.push_back(P.op_slot[i]);
+            continue;
+        }
         for (int o : outs_of[i]) {
             DaisInstr O{};
             O.kind = DK_OUTPUT, O.dst = o, O.a = P.op_slot[i], O.neg = out_negs[o] != 0;
@@ -282,6 +328,12 @@ inline int dais_shared_tile(int n_slots, long long budget) {
     const long long per_sample = 8LL * std::max(n_slots, 1);
     const long long t = std::min<long long>(256, budget / per_sample / 32 * 32);
     return (int)std::max<long long>(t, 0);
+}
+
+// Samples per launch of a profile run: at most `chunk`, a multiple of 256, and few enough that the per-warp records
+// (32 bytes per instruction and warp of 32 samples: n_instr bytes per sample) fit `record_bytes`.
+inline long long dais_profile_chunk(long long n_instr, long long chunk, long long record_bytes) {
+    return std::max<long long>(256, std::min(chunk, record_bytes / std::max(n_instr, 1LL) / 256 * 256));
 }
 
 } // namespace da

@@ -151,6 +151,19 @@ int da4ml_dais_info(const da4ml_dais_t *h, int64_t out[8]);
 int da4ml_dais_infer(da4ml_dais_t *h, const double *x, int64_t n_samples, double *y);
 /* the same with x and y in device memory (on the device the program was loaded on), on the library's stream */
 int da4ml_dais_infer_device(da4ml_dais_t *h, const double *x_dev, int64_t n_samples, double *y_dev);
+/* Profile of n_samples samples, every op (dead ones included) run as the reference runs them.  stats [4][n_ops]:
+ * min and max of each op's int64 value (INT64_MAX / INT64_MIN for no samples), the number of samples whose value lies
+ * outside the op's declared dtype range, and, for the wrapping ops (-1, +-2, +-3, +-6), the number of samples whose
+ * value the wrap step changed.  first = {sample, op} of the first value outside its range (sample order, then op
+ * order), {-1, -1} when there is none.  x in host memory; stats and first in host memory. */
+int da4ml_dais_profile(da4ml_dais_t *h, const double *x, int64_t n_samples, int64_t *stats, int64_t first[2]);
+/* the same with x in device memory, on the library's stream; stats and first are still host memory */
+int da4ml_dais_profile_device(da4ml_dais_t *h, const double *x_dev, int64_t n_samples, int64_t *stats, int64_t first[2]);
+/* The raw int64 values of ops[0..k) (each in [0, n_ops), duplicates allowed) for every sample: out [n_samples][k],
+ * the reference interpreter's buffer[op].  x and out in host memory. */
+int da4ml_dais_capture(da4ml_dais_t *h, const double *x, int64_t n_samples, const int32_t *ops, int32_t k, int64_t *out);
+/* the same with x and out in device memory (ops in host memory), on the library's stream */
+int da4ml_dais_capture_device(da4ml_dais_t *h, const double *x_dev, int64_t n_samples, const int32_t *ops, int32_t k, int64_t *out_dev);
 void da4ml_dais_free(da4ml_dais_t *h);
 /* Development switch, read by da4ml_dais_load: shared memory one CTA's slot file may use (a budget below 32 samples'
  * worth selects the global-memory regime) and samples per launch.  0 = automatic for either. */
