@@ -38,6 +38,7 @@ _L.da4ml_cmvm_plan.argtypes = [_i64p, C.c_int64, C.c_int, C.c_int, _i64p]
 _L.da4ml_cmvm_set_group_size.argtypes = [C.c_int]
 _L.da4ml_cmvm_set_accounting.argtypes = [C.c_int]
 _L.da4ml_cmvm_set_job_sharing.argtypes = [C.c_int]
+_L.da4ml_cmvm_set_first_attempt_caps.argtypes = [_i64p]
 _L.da4ml_cmvm_solve.argtypes = [_f32p, C.c_int64, C.c_int64, C.c_char_p, C.c_char_p, C.c_int, C.c_int, _f32p, _f32p, C.c_int, C.c_int, C.c_int, C.POINTER(_vp)]
 _L.da4ml_cmvm_solve_batch.argtypes = [C.c_int64, C.POINTER(_f32p), _i64p, _i64p, C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.POINTER(_f32p), C.POINTER(_f32p), C.c_int, C.c_int, C.c_int, C.POINTER(_vp)]
 _L.da4ml_cmvm_solve_batch_device.argtypes = [C.c_int64, C.POINTER(_vp), _i64p, _i64p, C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.POINTER(_f32p), C.POINTER(_f32p), C.c_int, C.c_int, C.c_int, C.POINTER(_vp)]
@@ -49,6 +50,7 @@ _L.da4ml_pipeline_stage_meta.argtypes = [_vp, C.c_int64, _i64p]
 _L.da4ml_pipeline_stage_copy.argtypes = [_vp, C.c_int64, _i64p, _i64p, _i64p, _i64p, _i64p, _f32p]
 _L.da4ml_pipeline_stage_counters.argtypes = [_vp, C.c_int64, _i64p]
 _L.da4ml_pipeline_stage_milestones.argtypes = [_vp, C.c_int64, _i64p]
+_L.da4ml_pipeline_stage_words.argtypes = [_vp, C.c_int64, _i64p]
 _L.da4ml_pipeline_device_ms.restype = C.c_double
 _L.da4ml_pipeline_device_ms.argtypes = [_vp]
 _L.da4ml_pipeline_launches.restype = C.c_int64
@@ -75,10 +77,11 @@ _L.da4ml_cmvm_cost_add.argtypes = [_f32p, _f32p, C.c_int64, C.c_int, C.c_int, C.
 
 EXPORTED_SYMBOLS = [
     'da4ml_cmvm_last_error', 'da4ml_cmvm_device_info', 'da4ml_cmvm_set_stream', 'da4ml_cmvm_set_group_size',
-    'da4ml_cmvm_set_accounting', 'da4ml_cmvm_set_job_sharing', 'da4ml_pipeline_profile', 'da4ml_cmvm_release', 'da4ml_cmvm_plan',
-    'da4ml_cmvm_solve', 'da4ml_cmvm_solve_batch', 'da4ml_cmvm_solve_batch_device', 'da4ml_cmvm_solve_single', 'da4ml_pipeline_free',
-    'da4ml_pipeline_n_stages', 'da4ml_pipeline_stage_meta', 'da4ml_pipeline_stage_copy',
-    'da4ml_pipeline_stage_counters', 'da4ml_pipeline_stage_milestones', 'da4ml_pipeline_device_ms', 'da4ml_pipeline_launches',
+    'da4ml_cmvm_set_accounting', 'da4ml_cmvm_set_job_sharing', 'da4ml_cmvm_set_first_attempt_caps', 'da4ml_pipeline_profile',
+    'da4ml_cmvm_release', 'da4ml_cmvm_plan', 'da4ml_cmvm_solve', 'da4ml_cmvm_solve_batch', 'da4ml_cmvm_solve_batch_device',
+    'da4ml_cmvm_solve_single', 'da4ml_pipeline_free', 'da4ml_pipeline_n_stages', 'da4ml_pipeline_stage_meta', 'da4ml_pipeline_stage_copy',
+    'da4ml_pipeline_stage_counters', 'da4ml_pipeline_stage_milestones', 'da4ml_pipeline_stage_words', 'da4ml_pipeline_device_ms',
+    'da4ml_pipeline_launches',
     'da4ml_cmvm_csd_decompose', 'da4ml_cmvm_int_arr_to_csd', 'da4ml_cmvm_kernel_decompose',
     'da4ml_cmvm_get_lsb_loc', 'da4ml_cmvm_iceil_log2', 'da4ml_cmvm_cost_add', 'da4ml_dais_run',
     'da4ml_dais_load', 'da4ml_dais_info', 'da4ml_dais_infer', 'da4ml_dais_infer_device', 'da4ml_dais_free',
@@ -148,6 +151,21 @@ def set_job_sharing(on: bool):
 def set_accounting(on: bool):
     """Exact work counters (sum over iterations of the live histogram size); slower, identical results."""
     _L.da4ml_cmvm_set_accounting(int(bool(on)))
+
+
+FIRST_ATTEMPT_CAPS = ['segment_entries_per_cta', 'list_rows_smem', 'spill_rows', 'log2_pair_counters', 'cells_per_cta', 'extra_expressions']
+
+
+def set_first_attempt_caps(**caps):
+    """Development switch: force capacities below the planner's choice on the first attempt of every round of
+    solve_single jobs (keywords from ``FIRST_ATTEMPT_CAPS``; omitted or 0 = the planner's value, no keywords = all
+    back to the planner).  Overflows are retried with the planner's sizes (``profile['retried_jobs']``); results do not
+    change.  ``plan()`` shows the first attempt's plan."""
+    unknown = set(caps) - set(FIRST_ATTEMPT_CAPS)
+    if unknown:
+        raise TypeError(f'unknown capacities: {sorted(unknown)}')
+    arr = np.asarray([int(caps.get(k, 0)) for k in FIRST_ATTEMPT_CAPS], np.int64)
+    _check(_L.da4ml_cmvm_set_first_attempt_caps(_ip(arr)))
 
 
 def _fp(a):
@@ -223,12 +241,16 @@ class RawPipeline:
                 ms = np.zeros(63, np.int64)
                 _check(_L.da4ml_pipeline_stage_milestones(handle, s, _ip(ms)))
                 cd['milestones'] = {250 << k: [int(v) for v in ms[9 * k : 9 * k + 9]] for k in range(7) if ms[9 * k + 8] > 0}
+                words = np.zeros(96, np.int64)
+                _check(_L.da4ml_pipeline_stage_words(handle, s, _ip(words)))
+                cd['split_passes'] = int(words[95])
                 self.counters.append(cd)
             self.device_ms = float(_L.da4ml_pipeline_device_ms(handle))
             self.launches = int(_L.da4ml_pipeline_launches(handle))
             prof = (C.c_double * 8)()
             _L.da4ml_pipeline_profile(handle, prof)
-            self.profile = dict(device_ms=prof[0], launches=int(prof[1]), solve_kernel_ms=prof[2], solve_kernel_launches=int(prof[3]), algo_bytes=prof[4], jobs_total=int(prof[5]), jobs_run=int(prof[6]))
+            self.profile = dict(device_ms=prof[0], launches=int(prof[1]), solve_kernel_ms=prof[2], solve_kernel_launches=int(prof[3]), algo_bytes=prof[4], jobs_total=int(prof[5]), jobs_run=int(prof[6]),
+                                retried_jobs=int(prof[7]))
         finally:
             _L.da4ml_pipeline_free(handle)
 

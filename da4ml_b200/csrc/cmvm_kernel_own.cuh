@@ -88,6 +88,7 @@ __device__ void solve_problem_own(const ProblemDesc &p, const Ctx &cx, const Own
         b.poll_iters = 0;
         ob.pool_used = 0;
         ob.pass_bits = 0;
+        ob.splits = 0;
         ob.n_ins = 0;
         ob.overflow = 0;
 #ifdef DA_RECOUNT_PROF
@@ -322,6 +323,8 @@ __device__ void solve_problem_own(const ProblemDesc &p, const Ctx &cx, const Own
         atomicAdd((unsigned long long *)&p.result_meta[META_R0], r0_cta);
         atomicAdd((unsigned long long *)&p.result_meta[META_RESCANNED], b.rescanned);
         atomicMax((long long *)&p.result_meta[META_LIST_MAX], (long long)b.list_max);
+        if (ob.splits)
+            atomicAdd((unsigned long long *)&p.result_meta[META_SPLITS], (unsigned long long)ob.splits);
         for (int k = 0; k < 8; ++k)
             atomicMax((long long *)&p.result_meta[META_PHASEMAX + k], b.phase[k]); // the slowest CTA's total per phase
         if (b.status != ST_OK)

@@ -341,6 +341,7 @@ int da4ml_cmvm_plan(const int64_t *jobs, int64_t n_jobs, int coop, int group_ove
         PlanEnv env;
         env.coop = coop;
         env.group_override = group_override;
+        std::copy(g_first_caps, g_first_caps + CAP_WORDS, env.caps); // (the first attempt's plan)
         const LaunchPlan P = plan_launch(pj, env);
         out[0] = P.cfg.G;
         out[1] = P.n_groups;
@@ -385,6 +386,19 @@ int da4ml_cmvm_set_job_sharing(int on) {
 int da4ml_cmvm_set_accounting(int on) {
     g_accounting = on;
     return DA4ML_OK;
+}
+int da4ml_cmvm_set_first_attempt_caps(const int64_t caps[6]) {
+    return guarded([&] {
+        if (!caps)
+            throw ApiError(DA4ML_E_INVALID, "da4ml_cmvm_set_first_attempt_caps: null caps");
+        for (int k = 0; k < CAP_WORDS; ++k)
+            if (caps[k] < 0 || caps[k] > INT32_MAX)
+                throw ApiError(DA4ML_E_INVALID, "da4ml_cmvm_set_first_attempt_caps: capacity " + std::to_string(k) + " out of range");
+        if (caps[CAP_HLOG] != 0 && (caps[CAP_HLOG] < HLOG_MIN || caps[CAP_HLOG] > HLOG_MAX))
+            throw ApiError(DA4ML_E_INVALID, "da4ml_cmvm_set_first_attempt_caps: log2_pair_counters must be 0 or " + std::to_string(HLOG_MIN) + ".." +
+                                                std::to_string(HLOG_MAX));
+        std::copy(caps, caps + CAP_WORDS, g_first_caps);
+    });
 }
 
 int da4ml_cmvm_solve_batch(
@@ -474,6 +488,7 @@ int da4ml_cmvm_solve_single(
         pl->solve_ms = tm.solve_ms;
         pl->solve_launches = tm.solve_launches;
         pl->algo_bytes = tm.algo_bytes;
+        pl->retried_jobs = tm.retried_jobs;
         *out = new da4ml_pipeline();
         (*out)->impl = std::move(pl);
     });
@@ -537,6 +552,12 @@ int da4ml_pipeline_stage_milestones(const da4ml_pipeline_t *p, int64_t s, int64_
     std::copy(p->impl->stages[s].counters + META_MILESTONES, p->impl->stages[s].counters + META_MILESTONES + 63, out);
     return DA4ML_OK;
 }
+int da4ml_pipeline_stage_words(const da4ml_pipeline_t *p, int64_t s, int64_t out[96]) {
+    if (!p || s < 0 || s >= (int64_t)p->impl->stages.size())
+        return DA4ML_E_INVALID;
+    std::copy(p->impl->stages[s].counters, p->impl->stages[s].counters + META_WORDS, out);
+    return DA4ML_OK;
+}
 double da4ml_pipeline_device_ms(const da4ml_pipeline_t *p) { return p ? p->impl->device_ms : 0.0; }
 int64_t da4ml_pipeline_launches(const da4ml_pipeline_t *p) { return p ? p->impl->launches : 0; }
 int da4ml_pipeline_profile(const da4ml_pipeline_t *p, double out[8]) {
@@ -549,7 +570,7 @@ int da4ml_pipeline_profile(const da4ml_pipeline_t *p, double out[8]) {
     out[4] = p->impl->algo_bytes;
     out[5] = (double)p->impl->jobs_total;
     out[6] = (double)p->impl->jobs_run;
-    out[7] = 0.0;
+    out[7] = (double)p->impl->retried_jobs;
     return DA4ML_OK;
 }
 

@@ -42,6 +42,7 @@ enum Meta : int {
     META_PHASE0 = 16, // 8 words: cycles spent by CTA rank 0 in substitute, recount, refresh, wait1, harvest, publish, wait2, collect
     META_PHASEMAX = 24, // 8 words: the same, maximum over the CTAs of the group
     META_MILESTONES = 32, // 7 x 9 words: cumulative phase cycles of CTA rank 0 (8 words) + cycles since the problem started, after 250 * 2^k greedy steps (k = 0..6)
+    META_SPLITS = 95,     // pair-counting passes abandoned for a full counter table and split in two (sum over the CTAs)
     META_WORDS = 96
 };
 

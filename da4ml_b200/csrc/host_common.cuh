@@ -25,6 +25,7 @@ static cudaStream_t g_stream = nullptr;
 static int g_group_override = 0;
 static int g_accounting = 0;
 static int g_share_jobs = 1;  // solve byte-identical solve_single jobs of one call once (host_solve.cuh)
+static long long g_first_caps[6] = {0}; // capacities forced on the first attempt of a round of jobs (host_plan.cuh FirstCap)
 
 struct ApiError : std::runtime_error {
     int code;
@@ -112,6 +113,7 @@ struct Timing {
     int64_t launches = 0;
     int64_t solve_launches = 0;
     double algo_bytes = 0;     // algorithmic bytes (SURVEY.md 8d) of every solve_single executed
+    int64_t retried_jobs = 0;  // jobs relaunched after a capacity overflow
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> pending;
     std::vector<char> is_solve;
     void mark_solve() { is_solve.back() = 1; }

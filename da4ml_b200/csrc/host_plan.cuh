@@ -19,11 +19,19 @@ struct PlanJob {
     int f_mul = 1, list_mul = 2; // capacity multipliers raised by retries
     int e_cap = 0;               // expression ids the job may use
 };
+// Capacities a development switch may force below the planner's choice on the first attempt of a round of jobs
+// (da4ml_cmvm_set_first_attempt_caps): small problems then take the spill, split-pass, compaction and retry paths.
+enum FirstCap : int { CAP_FSEG = 0, CAP_LCAP = 1, CAP_OVF = 2, CAP_HLOG = 3, CAP_POOL = 4, CAP_EXPR = 5, CAP_WORDS = 6 };
+// log2 of the pair-counter table: one owned expression has at most 3 rows x 63 shifts x 2 signs = 378 counters, which
+// must fit the 5/8 of the table one pass may claim (so a split always ends); slot indices are 16-bit
+constexpr int HLOG_MIN = 10, HLOG_MAX = 16;
+
 struct PlanEnv {
     int coop = 148;      // co-resident CTAs of the launch (one persistent 512-thread CTA per SM)
     bool accounting = false;
     int group_override = 0; // > 0: fixed group size (set_group_size)
     long long own_budget = 208 * 1024; // dynamic shared memory one CTA of the solve kernel may use
+    long long caps[CAP_WORDS] = {0};   // > 0: upper bound on that capacity of the final plan (the group size is chosen without them)
 };
 
 // shared-memory bytes of one CTA of the owner-partitioned kernel (mirrors own_plan in cmvm_kernel_own.cuh, which is the
@@ -74,6 +82,11 @@ inline LaunchPlan plan_for_group(const std::vector<PlanJob> &jobs, const PlanEnv
     }
     if (P.max_fcap >= (1LL << 27))
         P.max_fcap = (1LL << 27) - 1;
+    const long long *caps = env.caps;
+    if (caps[CAP_FSEG] > 0)
+        P.max_fcap = std::min(P.max_fcap, caps[CAP_FSEG]);
+    if (caps[CAP_POOL] > 0)
+        P.pool_cap = std::min(P.pool_cap, caps[CAP_POOL]);
     LaunchCfg &cfg = P.cfg;
     cfg.G = G;
     cfg.cpc = (P.n_out_max + G - 1) / G;
@@ -85,7 +98,8 @@ inline LaunchPlan plan_for_group(const std::vector<PlanJob> &jobs, const PlanEnv
     const long long budget = env.own_budget;
     P.narrow = (P.nbits_max <= 16 && (P.e_cap_max + G - 1) / G + 1 <= 65535) ? 1 : 0;
     // pair-counter hash table: as large as the target list capacity leaves room for (2^13 ... 2^11 counters)
-    for (int hlog = 13; hlog >= 11; --hlog) {
+    const int hlog_top = caps[CAP_HLOG] > 0 ? (int)std::min<long long>(13, caps[CAP_HLOG]) : 13;
+    for (int hlog = hlog_top; hlog >= std::min(11, hlog_top); --hlog) {
         const long long fixed = (long long)own_plan_bytes(cfg.nchunk_cap, P.n_out_max, P.e_cap_max, 0, hlog, P.narrow);
         long long lcap = (budget - fixed) / ((P.narrow ? 6LL : 12LL) * P.n_out_max);
         lcap = std::max<long long>(0, std::min(lcap, rows_hard)) & ~1LL;
@@ -96,14 +110,21 @@ inline LaunchPlan plan_for_group(const std::vector<PlanJob> &jobs, const PlanEnv
             break;
     }
     P.roomy = P.lists_fit && P.hlog >= 12; // (a 2048-counter table means many counting passes per step while the rows are dense)
+    if (caps[CAP_LCAP] > 0) // (the rows taken out of shared memory become spill rows)
+        P.lcap = (int)(std::min<long long>(P.lcap, caps[CAP_LCAP]) & ~1LL);
     P.ovf_cap = std::max<long long>(0, rows_hard - P.lcap);
+    if (caps[CAP_OVF] > 0)
+        P.ovf_cap = std::min(P.ovf_cap, caps[CAP_OVF]);
     P.smem_bytes = own_plan_bytes(cfg.nchunk_cap, P.n_out_max, P.e_cap_max, P.lcap, P.hlog, P.narrow);
     return P;
 }
 
 // Group size: as many concurrent problems as possible, but with the owner lists in shared memory -- the jobs then run
 // in equal waves over coop / G groups.
-inline LaunchPlan plan_launch(const std::vector<PlanJob> &jobs, const PlanEnv &env) {
+inline LaunchPlan plan_launch(const std::vector<PlanJob> &jobs, const PlanEnv &env_caps) {
+    PlanEnv env = env_caps; // (forced capacities apply to the final plan only: they do not change the group size)
+    for (long long &c : env.caps)
+        c = 0;
     const int n = (int)jobs.size(), coop = env.coop;
     long long want = 1; // CTAs one problem can keep busy
     for (const PlanJob &j : jobs) {
@@ -138,7 +159,7 @@ inline LaunchPlan plan_launch(const std::vector<PlanJob> &jobs, const PlanEnv &e
     }
     if (env.group_override > 0)
         G = std::min(env.group_override, coop);
-    LaunchPlan P = plan_for_group(jobs, env, G);
+    LaunchPlan P = plan_for_group(jobs, env_caps, G);
     P.n_groups = std::max(1, std::min(n, coop / G));
     return P;
 }

@@ -16,6 +16,7 @@ struct PipelineImpl {
     double device_ms = 0, solve_ms = 0, algo_bytes = 0;
     int64_t launches = 0, solve_launches = 0;
     int64_t jobs_total = 0, jobs_run = 0; // solve_single jobs the reference would execute / executed after sharing identical ones
+    int64_t retried_jobs = 0;             // jobs relaunched after a capacity overflow
 };
 
 struct Candidate {
@@ -479,6 +480,7 @@ static void solve_many(
         pl->algo_bytes = tm.algo_bytes;
         pl->jobs_total = jobs_total;
         pl->jobs_run = jobs_run;
+        pl->retried_jobs = tm.retried_jobs;
     }
 }
 

@@ -203,6 +203,7 @@ static void run_stage_jobs(std::vector<StageJob *> &jobs, Timing &tm, bool want_
         };
         std::vector<OOff> oo(n);
         long long max_cols = 0, max_colcap = 0, max_heap = 0, max_ecap = 0;
+        const long long *caps = attempt == 0 ? g_first_caps : nullptr; // forced capacities (set_first_attempt_caps): first attempt only
         for (int i = 0; i < n; ++i) {
             StageJob &j = *todo[i];
             const int *pm = &pmeta[(size_t)i * PM_WORDS];
@@ -210,6 +211,8 @@ static void run_stage_jobs(std::vector<StageJob *> &jobs, Timing &tm, bool want_
             const long long d0 = pm[PM_D0];
             d.nbits = pm[PM_NBITS];
             long long t_cap = j.full_expr ? d0 : std::min<long long>(d0, d0 / 2 + 1024);
+            if (caps && caps[CAP_EXPR] > 0)
+                t_cap = std::min(t_cap, caps[CAP_EXPR]);
             d.e_cap = (int)(j.n_in + t_cap + 1);
             d.ops_cap = (int)(j.n_in + d0 + 1);
             d.col_cap = pm[PM_COLCAP] + 1;
@@ -252,6 +255,8 @@ static void run_stage_jobs(std::vector<StageJob *> &jobs, Timing &tm, bool want_
         penv.accounting = accounting;
         penv.own_budget = g_own_smem_max - 1024;
         penv.group_override = g_group_override;
+        if (caps)
+            std::copy(caps, caps + CAP_WORDS, penv.caps);
         const LaunchPlan plan = plan_launch(pj, penv);
         const LaunchCfg cfg = plan.cfg;
         const int G = cfg.G, n_groups = plan.n_groups;
@@ -494,6 +499,7 @@ static void run_stage_jobs(std::vector<StageJob *> &jobs, Timing &tm, bool want_
                 memcpy(j.trace, dp + dof[i].tr, sizeof(int) * 5 * (size_t)rows);
             }
         }
+        tm.retried_jobs += (int64_t)again.size();
         todo.swap(again);
     }
     if (!todo.empty())

@@ -47,6 +47,7 @@ struct OwnBlock {
     int grew;        // a subset had to be split in this step
     int ins_max;     // most slots claimed by one pass of this step
     int sub_top;
+    int splits;      // counting passes abandoned and split in two (whole problem)
 #ifdef DA_RECOUNT_PROF
     long long xphase[4], xt; // development build: cycles of thread 0 in the parts of the recount (setup, counting, harvest)
 #endif
@@ -759,6 +760,7 @@ __device__ void own_recount(const ProblemDesc &p, const Ctx &cx, const OwnCtx &o
                     ob.sub_stack[ob.sub_top++] = ((uint32_t)(bits + 1) << 16) | (val | (1u << bits));
                     ob.sub_stack[ob.sub_top++] = ((uint32_t)(bits + 1) << 16) | val;
                     ob.grew = 1;
+                    ob.splits += 1;
                 }
             }
             else

@@ -61,6 +61,14 @@ int da4ml_cmvm_set_accounting(int on);
  * pure function of its inputs, so by default identical jobs are solved once and the result shared (identical output to
  * the reference, which solves each candidate separately).  0 switches the sharing off. */
 int da4ml_cmvm_set_job_sharing(int on);
+/* Development switch for testing the solver's capacity paths: caps = {segment_entries_per_cta, list_rows_smem,
+ * spill_rows, log2_pair_counters, cells_per_cta, extra_expressions} (the fields of da4ml_cmvm_plan plus the expressions
+ * a job may create beyond its inputs).  0 keeps the planner's value.  A nonzero value replaces the planner's only on the
+ * first attempt of each round of solve_single jobs and only when it is smaller; shared-memory rows taken away become
+ * spill rows.  A job that overflows a forced capacity reports it and is relaunched with the planner's escalated sizes
+ * (counted in da4ml_pipeline_profile slot 7), so results do not change.  da4ml_cmvm_plan shows the first attempt's
+ * plan.  Negative values and log2_pair_counters outside 10..16 give DA4ML_E_INVALID.  All zero by default. */
+int da4ml_cmvm_set_first_attempt_caps(const int64_t caps[6]);
 
 /* ---- solve -------------------------------------------------------------------------------------
  * Replaces `solve` (bindings.cc:184-225 -> api.cc:147-250).
@@ -122,12 +130,16 @@ int da4ml_pipeline_stage_counters(const da4ml_pipeline_t *p, int64_t stage, int6
  * problem's group spent in each of the 8 phases of a greedy step, and the cycles since the loop started (zero for
  * milestones the stage did not reach). */
 int da4ml_pipeline_stage_milestones(const da4ml_pipeline_t *p, int64_t stage, int64_t out[63]);
+/* All 96 result words of one stage (enum Meta in csrc/cmvm_types.cuh): the 32 counters, the 63 milestone words and word
+ * 95, the number of pair-counting passes that ran out of counters and were split in two. */
+int da4ml_pipeline_stage_words(const da4ml_pipeline_t *p, int64_t stage, int64_t out[96]);
 /* Device milliseconds spent in this library's kernels for the call that produced p (CUDA events). */
 double da4ml_pipeline_device_ms(const da4ml_pipeline_t *p);
 /* Number of kernel launches issued for the call that produced p. */
 int64_t da4ml_pipeline_launches(const da4ml_pipeline_t *p);
 /* Profile of the call that produced p: {device_ms, launches, solve_kernel_ms, solve_kernel_launches,
- * algorithmic_bytes (all solve_single jobs of the call, exact in accounting mode), 0, 0, 0}. */
+ * algorithmic_bytes (all solve_single jobs of the call, exact in accounting mode), jobs_total, jobs_run (solve_single
+ * jobs of the reference / after sharing identical ones), retried_jobs (relaunches after a capacity overflow)}. */
 int da4ml_pipeline_profile(const da4ml_pipeline_t *p, double out[8]);
 
 /* ---- DAIS replay (SURVEY 8f N2) -------------------------------------------------------------------

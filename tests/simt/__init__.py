@@ -47,6 +47,7 @@ def lib():
         L.sim_set_wide_rows.argtypes = [C.c_int]
         L.sim_set_segment_cap.argtypes = [C.c_int]
         L.sim_set_caps.argtypes = [C.c_int, C.c_int]
+        L.sim_set_first_attempt_caps.argtypes = [C.POINTER(C.c_longlong)]
         L.sim_kernel_decompose.argtypes = [FP, C.c_int, C.c_int, C.c_int, FP, FP]
         _lib = L
     return _lib
@@ -71,6 +72,15 @@ def set_list_cap(rows: int | None):
 def set_wide_rows(on: bool):
     """Keep three words per shared-memory list row even when 6 bytes would do."""
     lib().sim_set_wide_rows(int(bool(on)))
+
+
+def set_first_attempt_caps(**caps):
+    """The product's first-attempt capacities (``da4ml_b200._binary.FIRST_ATTEMPT_CAPS``; omitted = planner's), applied
+    to the plan and the expression table as the host driver applies them on a first attempt (no retry here)."""
+    names = ['segment_entries_per_cta', 'list_rows_smem', 'spill_rows', 'log2_pair_counters', 'cells_per_cta', 'extra_expressions']
+    arr = (C.c_longlong * 6)(*[int(caps.pop(k, 0)) for k in names])
+    assert not caps, f'unknown capacities: {sorted(caps)}'
+    lib().sim_set_first_attempt_caps(arr)
 
 
 def set_own_caps(hash_log: int = 0, spill_rows: int = -1, list_rows: int | None = None):

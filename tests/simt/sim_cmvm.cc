@@ -64,6 +64,12 @@ void sim_set_list_cap(int rows) {
     g_lcap_override = rows < 0 ? 0 : rows;
     g_lcap_set = rows >= 0;
 }
+// the product's first-attempt capacities (host_plan.cuh FirstCap; 0 = planner's), applied where run_stage_jobs applies them
+static long long g_first_caps[CAP_WORDS] = {0};
+void sim_set_first_attempt_caps(const long long *caps) {
+    for (int k = 0; k < CAP_WORDS; ++k)
+        g_first_caps[k] = caps[k];
+}
 // log2 of the pair-counter hash table (0 = planner's), spill rows per owner list (< 0 = planner's)
 void sim_set_wide_rows(int on) { g_wide_rows = on; } // 12-byte list rows even when 6 bytes would do
 void sim_set_own_caps(int hlog, int ovf_rows) {
@@ -181,7 +187,9 @@ static void run_jobs(std::vector<SimJob> &jobs, int G, int n_groups, int cta_thr
         const int *pm = d.prep_meta;
         const long long d0 = pm[PM_D0];
         d.nbits = pm[PM_NBITS];
-        const long long t_cap = std::min<long long>(d0, d0 / 2 + 1024);
+        long long t_cap = std::min<long long>(d0, d0 / 2 + 1024);
+        if (g_first_caps[CAP_EXPR] > 0)
+            t_cap = std::min(t_cap, g_first_caps[CAP_EXPR]);
         d.e_cap = (int)(j.n_in + t_cap + 1);
         d.ops_cap = (int)(j.n_in + d0 + 1);
         d.col_cap = pm[PM_COLCAP] + 1;
@@ -215,6 +223,7 @@ static void run_jobs(std::vector<SimJob> &jobs, int G, int n_groups, int cta_thr
     env.coop = G * n_groups;
     env.group_override = G;
     env.accounting = accounting;
+    std::copy(g_first_caps, g_first_caps + CAP_WORDS, env.caps);
     LaunchPlan plan = plan_launch(pj, env);
     if (g_lcap_set) { // shrink the shared-memory part of the owner lists: rows spill to global memory
         plan.ovf_cap += std::max(0, plan.lcap - g_lcap_override);
